@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            # this repo, N ranks (torchrun for N > 1)
     python bench.py --impl reference --steps K --warmup W    # the unmodified reference modules on the host cores
     python bench.py --res 128 --strong --gpus N              # BASELINE configs[3]: 8 grids in total, 8/N per GPU
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   # also write the outputs of the last timed step
 
 A "step" is one denoising step of pc_sampler for one batch: U-Net evaluation + ancestral update over
 [batch, 4, 64, 64, 64]. metric = sample-steps/s = batch * steps / time, whole job (sum over ranks).
@@ -35,6 +36,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 METRIC = "denoising sample-steps/sec at res-64 (4x64^3), uncond_gen PC sampler"
@@ -139,8 +141,10 @@ class Ctx:
         return t.item()
 
 
-def sampler_leg(ctx, precision, B, R, K, W, dump_profile=None, full_run=False):
-    """One operand mode: device-resident loop, end-to-end loop, roofline of the GEMM launches, clocks."""
+def sampler_leg(ctx, precision, B, R, K, W, dump_profile=None, full_run=False, dump_outputs=False):
+    """One operand mode: device-resident loop, end-to-end loop, roofline of the GEMM launches, clocks. With `dump_outputs`
+    the leg also returns what the last timed step of the device-resident loop left for its caller (the state x and
+    x_mean), sampled by `output_sample`."""
     from meshdiffusion_b200.diffusion import sde_lib, sampling
     from meshdiffusion_b200.geometry.dmtet import grid_mask_from_tets
     device, world, rank = ctx.device, ctx.world, ctx.rank
@@ -152,9 +156,12 @@ def sampler_leg(ctx, precision, B, R, K, W, dump_profile=None, full_run=False):
     mask_flat = mask.reshape(-1).contiguous()
     timesteps = torch.linspace(sde.T, 1e-3, sde.N, device=device)
     idx = (timesteps * (sde.N - 1)).long()
-    labels_all = (timesteps * (sde.N - 1)).cpu().tolist()
-    betas = sde.discrete_betas[idx].cpu().tolist()
-    stds = sde.sqrt_1m_alphas_cumprod[idx].cpu().tolist()
+    # a window of more than N steps runs on into the schedule again from its first step, so --warmup + --steps can be
+    # any length
+    cyclic = lambda v: [v[i % len(v)] for i in range(max(len(v), W + K))]
+    labels_all = cyclic((timesteps * (sde.N - 1)).cpu().tolist())
+    betas = cyclic(sde.discrete_betas[idx].cpu().tolist())
+    stds = cyclic(sde.sqrt_1m_alphas_cumprod[idx].cpu().tolist())
     g = torch.Generator(device=device).manual_seed(42 + rank)
     x = (torch.randn(B, 4, R, R, R, device=device, generator=g) * mask).contiguous()
 
@@ -166,14 +173,17 @@ def sampler_leg(ctx, precision, B, R, K, W, dump_profile=None, full_run=False):
     ctx.barrier()
     clocks = ClockSampler(ctx.local)
     clocks.start()
-    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    e0.record()
-    native_steps(W, K)
-    e1.record()
-    ctx.barrier()
+    try:
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        x_mean = native_steps(W, K)
+        e1.record()
+        ctx.barrier()
+    finally:
+        clk = clocks.stop()
     ms = ctx.max_over_ranks(e0.elapsed_time(e1))
-    clk = clocks.stop()
     value = world * B * K / (ms * 1e-3)
+    outputs = {f"{precision}_x": output_sample(x), f"{precision}_x_mean": output_sample(x_mean)} if dump_outputs else None
 
     # ---- the complete 999-evaluation run (opt-in: minutes), so samples/s is measured rather than extrapolated
     full = None
@@ -249,7 +259,17 @@ def sampler_leg(ctx, precision, B, R, K, W, dump_profile=None, full_run=False):
     net.release_engine()
     del model, net
     torch.cuda.empty_cache()
-    return leg, mask
+    return leg, mask, outputs
+
+
+def output_sample(t, n=1 << 21):
+    """float32 copy of at most `n` elements of `t`: all of them, or a fixed seeded sample (sorted flat indices, the same for
+    every run and build) of a larger tensor. 2^21 elements keep the six arrays of three operand modes at 48 MB."""
+    flat = t.detach().reshape(-1)
+    if flat.numel() > n:
+        idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:n].sort().values
+        flat = flat[idx.to(flat.device)]
+    return flat.float().cpu().numpy()
 
 
 def ncu_traffic(precision):
@@ -303,10 +323,12 @@ def run_ours(args):
             raise SystemExit(f"--strong: {B} grids do not divide over {ctx.world} ranks")
         B //= ctx.world
     precisions = [args.precision] + [p for p in args.legs.split(",") if p and p != args.precision]
-    legs, mask = {}, None
+    legs, mask, outputs = {}, None, {}
     for i, prec in enumerate(precisions):
-        legs[prec], mask = sampler_leg(ctx, prec, B, R, K, W, dump_profile=args.dump_profile if i == 0 else None,
-                                       full_run=args.full_run and i == 0)
+        legs[prec], mask, out = sampler_leg(ctx, prec, B, R, K, W, dump_profile=args.dump_profile if i == 0 else None,
+                                            full_run=args.full_run and i == 0, dump_outputs=bool(args.dump_outputs) and ctx.rank == 0)
+        if out:
+            outputs.update(out)
         if ctx.rank == 0:  # progress on stderr (stdout carries only the final JSON line)
             print(f"[bench] {prec}: value {legs[prec]['value']:.2f} e2e {legs[prec]['e2e']['value']:.2f} {UNIT}, "
                   f"gemm frac {legs[prec]['roofline']['frac']:.3f}", file=sys.stderr, flush=True)
@@ -360,6 +382,10 @@ def run_ours(args):
             "engine": head["engine"], "full_run": head["full_run"], "train": train,
         }
         print(json.dumps(line))
+    if outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if ctx.dist is not None:
         ctx.dist.destroy_process_group()
 
@@ -413,7 +439,13 @@ def main():
     ap.add_argument("--no-torch-gpu-baseline", action="store_true")
     ap.add_argument("--no-train-leg", action="store_true", help="skip the training-step measurement (tools/bench_train.py)")
     ap.add_argument("--dump-profile", default=None, help="write the per-launch CUDA-event times of one forward as JSON")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last timed step of each operand mode's device-resident loop returned (rank 0: state x "
+                         "and x_mean) as DIR/<mode>_x.npy and DIR/<mode>_x_mean.npy, float32, a fixed seeded sample of at "
+                         "most 2^21 elements each; the inputs depend only on the arguments, so two builds compare output for output")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.batch is None:
         args.batch = 8 if args.res == 128 else 32
     if args.legs is None:

@@ -1,82 +1,38 @@
 """CPU: checkpoints interchange with the REFERENCE's own code in both directions (the drop-in contract of SURVEY 8b:
 `torch.save({'optimizer','model','ema','step'})` with `module.`-prefixed model keys, positional EMA shadow list, the stock
-Adam state). The reference side runs in a subprocess from baseline/_ref (its `lib.diffusion.utils.restore_checkpoint` /
-`save_checkpoint`, `DDPMRes64` inside `nn.DataParallel`, `ExponentialMovingAverage`, `losses.get_optimizer`); nothing of this
-package is imported there."""
+Adam state). oracle/make_host_golden.py stores, from the reference's code, what its `lib.diffusion.utils.restore_checkpoint`
+loads into -- the state dict of `DDPMRes64` inside `nn.DataParallel`, the parameter list that `ExponentialMovingAverage`
+and `losses.get_optimizer`'s Adam follow (tests/golden/reference_host.json.xz) -- and a checkpoint its `save_checkpoint` wrote
+(tests/golden/reference_checkpoint_tiny.pth.xz)."""
+import json
+import lzma
 import os
-import subprocess
-import sys
+import shutil
 
-import pytest
 import torch
 
-from helpers import ROOT, tiny_config
-
-REF_SIDE = r'''
-import os, sys, torch
-root, ours_ckpt, ours_plain, ref_ckpt, ref_plain = sys.argv[1:6]
-sys.path.insert(0, root)
-from baseline import reference_arm
-ref, config = reference_arm.load("cpu")
-import lib.diffusion.utils as rutils, lib.diffusion.losses as rlosses
-from lib.diffusion.models.ema import ExponentialMovingAverage
-config.data.image_size, config.model.nf, config.model.ch_mult = 16, 32, (1, 2)
-config.model.num_res_blocks, config.model.attn_resolutions = 1, (8,)
-
-def fresh(seed):
-    torch.manual_seed(seed)
-    model = ref["mutils"].create_model(config)            # models/utils.py:88-96 -> nn.DataParallel shell, `module.` keys
-    ema = ExponentialMovingAverage(model.parameters(), decay=config.model.ema_rate)
-    opt = rlosses.get_optimizer(config, model.parameters())
-    return dict(optimizer=opt, model=model, ema=ema, step=0)
-
-# (1) a checkpoint written by meshdiffusion_b200 restores through the reference's restore_checkpoint
-state = rutils.restore_checkpoint(ours_ckpt, fresh(1), "cpu")
-plain = torch.load(ours_plain, map_location="cpu")
-assert state["step"] == plain["step"], (state["step"], plain["step"])
-sd = state["model"].state_dict()
-assert set(sd) == set(plain["model"]), set(sd) ^ set(plain["model"])
-for k, v in plain["model"].items():
-    assert sd[k].dtype == v.dtype and torch.equal(sd[k], v), k
-assert state["ema"].num_updates == plain["ema_num_updates"] and state["ema"].decay == plain["ema_decay"]
-for a, b in zip(state["ema"].shadow_params, plain["ema_shadow"]):
-    assert torch.equal(a, b)
-ost = state["optimizer"].state_dict()
-assert len(ost["state"]) == len(plain["opt_state"])
-for i, s in plain["opt_state"].items():
-    for f in ("exp_avg", "exp_avg_sq"):
-        assert torch.equal(ost["state"][i][f], s[f]), (i, f)
-    assert float(ost["state"][i]["step"]) == float(s["step"])
-# the restored reference optimiser keeps stepping (its state is the stock Adam layout)
-for p in state["model"].parameters():
-    p.grad = torch.zeros_like(p)
-state["optimizer"].step()
-print("REF_RESTORED_OURS", len(sd), len(ost["state"]))
-
-# (2) a checkpoint written by the reference: one Adam step on seeded gradients + two EMA updates, its own save_checkpoint
-st = fresh(2)
-g = torch.Generator().manual_seed(3)
-for p in st["model"].parameters():
-    p.grad = torch.randn(p.shape, generator=g) * 1e-2
-st["optimizer"].step()
-st["ema"].update(st["model"].parameters())
-st["ema"].update(st["model"].parameters())
-st["step"] = 11
-rutils.save_checkpoint(ref_ckpt, st)
-torch.save({"model": {k: v.clone() for k, v in st["model"].state_dict().items()},
-            "ema_shadow": [t.clone() for t in st["ema"].shadow_params], "ema_num_updates": st["ema"].num_updates,
-            "opt_state": {i: {k: (v.clone() if torch.is_tensor(v) else v) for k, v in s.items()}
-                          for i, s in st["optimizer"].state_dict()["state"].items()},
-            "param_groups": st["optimizer"].state_dict()["param_groups"]}, ref_plain)
-print("REF_SAVED", len(st["model"].state_dict()))
-'''
+from helpers import GOLD, tiny_config
 
 
-def _have_reference():
-    return os.path.exists(os.path.join(ROOT, "baseline", "_ref", "lib", "diffusion", "utils.py"))
+def _restore_as_the_reference(path, layout):
+    """What the reference's restore_checkpoint (utils.py:6-20) does with `path` on CPU, over a state of its layout:
+    torch.load, Adam.load_state_dict, model.load_state_dict(strict=False), EMA.load_state_dict (attribute copy)."""
+    loaded = torch.load(path, map_location="cpu")
+    assert {"optimizer", "model", "ema", "step"} <= set(loaded)
+    model = {k: (shape, dtype) for k, shape, dtype in layout["model"]}
+    for k, v in loaded["model"].items():  # strict=False skips unknown keys, but a shape mismatch still raises
+        if k in model:
+            assert list(v.shape) == model[k][0], (k, list(v.shape), model[k][0])
+    params = [torch.nn.Parameter(torch.zeros(shape), requires_grad=rg) for shape, rg in layout["parameters"]]
+    hyper = {k: (tuple(v) if isinstance(v, list) else v) for k, v in layout["param_groups"][0].items() if k != "params"}
+    opt = torch.optim.Adam(params, **hyper)
+    opt.load_state_dict(loaded["optimizer"])
+    assert set(layout["ema_fields"]) <= set(loaded["ema"])
+    shadow = loaded["ema"]["shadow_params"]
+    assert [list(t.shape) for t in shadow] == [shape for shape, rg in layout["parameters"] if rg]
+    return loaded, model, opt, params
 
 
-@pytest.mark.skipif(not _have_reference(), reason="baseline/_ref not staged (python baseline/install_reference.py)")
 def test_checkpoints_interchange_with_the_reference_code(tmp_path):
     from meshdiffusion_b200.diffusion import losses
     from meshdiffusion_b200.diffusion.models import utils as mutils
@@ -105,23 +61,42 @@ def test_checkpoints_interchange_with_the_reference_code(tmp_path):
                             "exp_avg_sq": torch.rand(p.shape, generator=g)}
     st["ema"].update(st["model"].parameters())
     st["step"] = 7
-    ours_ckpt, ours_plain = str(tmp_path / "ours.pth"), str(tmp_path / "ours_plain.pt")
-    ref_ckpt, ref_plain = str(tmp_path / "ref.pth"), str(tmp_path / "ref_plain.pt")
+    ours_ckpt = str(tmp_path / "ours.pth")
     save_checkpoint(ours_ckpt, st)
-    torch.save({"model": {k: v.clone() for k, v in st["model"].state_dict().items()}, "step": 7,
-                "ema_shadow": [t.clone() for t in st["ema"].shadow_params], "ema_num_updates": st["ema"].num_updates,
-                "ema_decay": st["ema"].decay,
-                "opt_state": {i: {k: v.clone() for k, v in s.items()} for i, s in opt.state_dict()["state"].items()}}, ours_plain)
+    plain = {"model": {k: v.clone() for k, v in st["model"].state_dict().items()},
+             "ema_shadow": [t.clone() for t in st["ema"].shadow_params], "ema_num_updates": st["ema"].num_updates,
+             "ema_decay": st["ema"].decay,
+             "opt_state": {i: {k: v.clone() for k, v in s.items()} for i, s in opt.state_dict()["state"].items()}}
 
-    env = dict(os.environ, OMP_NUM_THREADS="4")
-    r = subprocess.run([sys.executable, "-c", REF_SIDE, ROOT, ours_ckpt, ours_plain, ref_ckpt, ref_plain], capture_output=True,
-                       text=True, env=env, timeout=600)
-    assert r.returncode == 0, r.stdout + r.stderr
-    assert "REF_RESTORED_OURS" in r.stdout and "REF_SAVED" in r.stdout
+    # ---- the file -> the reference's restore_checkpoint
+    layout = json.load(lzma.open(os.path.join(GOLD, "reference_host.json.xz"), "rt"))["checkpoint_layout"]
+    loaded, model, ropt, rparams = _restore_as_the_reference(ours_ckpt, layout)
+    assert loaded["step"] == 7
+    assert set(model) == set(plain["model"]), set(model) ^ set(plain["model"])
+    for k, v in plain["model"].items():
+        assert model[k][1] == str(v.dtype) and torch.equal(loaded["model"][k], v), k
+    assert loaded["ema"]["num_updates"] == plain["ema_num_updates"] and loaded["ema"]["decay"] == plain["ema_decay"]
+    for a, b in zip(loaded["ema"]["shadow_params"], plain["ema_shadow"]):
+        assert torch.equal(a, b)
+    ost = ropt.state_dict()
+    assert len(ost["state"]) == len(plain["opt_state"])
+    for i, s in plain["opt_state"].items():
+        for f in ("exp_avg", "exp_avg_sq"):
+            assert torch.equal(ost["state"][i][f], s[f]), (i, f)
+        assert float(ost["state"][i]["step"]) == float(s["step"])
+    # the restored reference optimiser keeps stepping (its state is the stock Adam layout)
+    for p in rparams:
+        p.grad = torch.zeros_like(p)
+    ropt.step()
 
     # ---- the reference's file -> ours
+    ref_ckpt = str(tmp_path / "ref.pth")
+    with lzma.open(os.path.join(GOLD, "reference_checkpoint_tiny.pth.xz"), "rb") as src, open(ref_ckpt, "wb") as dst:
+        shutil.copyfileobj(src, dst)
+    raw = torch.load(ref_ckpt, map_location="cpu")
+    plain = {"model": raw["model"], "ema_shadow": raw["ema"]["shadow_params"], "ema_num_updates": raw["ema"]["num_updates"],
+             "opt_state": raw["optimizer"]["state"], "param_groups": raw["optimizer"]["param_groups"]}
     st2 = restore_checkpoint(ref_ckpt, fresh(8), "cpu")
-    plain = torch.load(ref_plain, map_location="cpu", weights_only=False)
     assert st2["step"] == 11
     sd = st2["model"].state_dict()
     assert set(sd) == set(plain["model"])

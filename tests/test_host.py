@@ -1,6 +1,8 @@
 """CPU: host-side logic -- parameter table vs the reference's state_dict, checkpoint layout, config surface, CLI,
 registries, EMA arithmetic, and a world_size-2 gloo run of the batch-sharded sampler plumbing."""
+import hashlib
 import json
+import lzma
 import os
 import subprocess
 import sys
@@ -270,10 +272,9 @@ def test_on_device_augmentation_matches_items(tmp_path):
 
 
 def test_partial_dmtet_and_grid_producers():
-    """geometry/formats.py against the reference's own code: data/tets_to_3dgrid.py::tet_to_grids exec'd from source, and the
-    fit_singleview.py:798-827 visibility tail restated literally."""
+    """geometry/formats.py against the reference's own code: data/tets_to_3dgrid.py::tet_to_grids (its output pinned by a
+    digest), and the fit_singleview.py:798-827 visibility tail restated literally."""
     from meshdiffusion_b200.geometry import dmtet, formats
-    ref_root = "/root/reference"
     verts, idx = dmtet.load_tet_grid(64)
     coords = dmtet.grid_coords_of_tet_vertices(verts)
     g = torch.Generator().manual_seed(3)
@@ -285,12 +286,9 @@ def test_partial_dmtet_and_grid_producers():
     x, y, z = coords[:, 0], coords[:, 1], coords[:, 2]
     assert torch.equal(grid[0, x, y, z], sdf) and torch.equal(grid[1:, x, y, z], deform.t())
     assert torch.equal(grid.abs().sum(0) != 0, dmtet.grid_mask_from_tets(64) == 1)  # sdf is +-1 on every tet vertex
-    if os.path.exists(os.path.join(ref_root, "data/tets_to_3dgrid.py")):  # authoring container: the reference function itself
-        src = open(os.path.join(ref_root, "data/tets_to_3dgrid.py")).read().split("if __name__")[0]
-        ns = {}
-        exec(src, ns)
-        want = ns["tet_to_grids"](coords, (sdf.unsqueeze(-1), deform), 64)
-        assert torch.equal(grid, want)
+    # the reference function itself on the same inputs, as its sha256 (oracle/make_host_golden.py)
+    want = json.load(lzma.open(os.path.join(GOLD, "reference_host.json.xz"), "rt"))["tet_to_grids_sha256"]
+    assert hashlib.sha256(grid.contiguous().numpy().tobytes()).hexdigest() == want
     # visibility -> dmtet.pt
     vis_id = torch.randperm(Fn, generator=g)[:5000]
     rast_id = torch.randperm(Fn, generator=g)[:300]

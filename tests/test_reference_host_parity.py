@@ -1,102 +1,21 @@
-"""CPU: host-side pieces of the drop-in surface compared with the REFERENCE's own code (baseline/_ref, run in a subprocess so
-its `configs` / `lib` packages never meet this repository's): config trees key by key, registered predictor / corrector /
+"""CPU: host-side pieces of the drop-in surface compared with what the REFERENCE's own code computes (stored in
+tests/golden/reference_host.json.xz by oracle/make_host_golden.py): config trees key by key, registered predictor / corrector /
 model names, the VP-SDE tables and `marginal_prob`, the EMA recursion, the optimiser construction and the warm-up / clip
 arithmetic of `optimization_manager` (lib/diffusion/losses.py:26-52)."""
 import json
+import lzma
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-from helpers import ROOT
-
-REF_SIDE = r'''
-import json, sys, torch
-root, out = sys.argv[1:3]
-sys.path.insert(0, root)
-from baseline import reference_arm
-ref, config = reference_arm.load("cpu")
-import importlib
-from configs import res128 as cfg128
-import lib.diffusion.losses as rlosses
-from lib.diffusion.models.ema import ExponentialMovingAverage
-
-def flat(c, pre=""):
-    o = {}
-    for k, v in c.items():
-        if k == "device":
-            continue
-        if isinstance(v, dict):
-            o.update(flat(v, pre + k + "."))
-        else:
-            o[pre + k] = list(v) if isinstance(v, tuple) else v
-    return o
-
-res = {"res64": flat(config), "res128": flat(cfg128.get_config())}
-samp = ref["sampling"]
-res["predictors"] = sorted(samp._PREDICTORS)
-res["correctors"] = sorted(samp._CORRECTORS)
-res["models"] = sorted(ref["mutils"]._MODELS)
-sde = ref["sde_lib"].VPSDE(beta_min=config.model.beta_min, beta_max=config.model.beta_max, N=config.model.num_scales)
-tables = {n: getattr(sde, n).double().tolist() for n in ("discrete_betas", "alphas", "alphas_cumprod", "sqrt_alphas_cumprod", "sqrt_1m_alphas_cumprod")}
-x = torch.linspace(-1, 1, 24).view(2, 3, 4)
-t = torch.tensor([0.25, 0.9])
-mean, std = sde.marginal_prob(x, t)
-tables["mp_mean"], tables["mp_std"] = mean.double().tolist(), std.double().tolist()
-res["sde"] = tables
-# EMA recursion (ema.py:43-64): three updates of a moving parameter
-p = [torch.nn.Parameter(torch.arange(6, dtype=torch.float32))]
-ema = ExponentialMovingAverage(p, decay=0.9999)
-trace = []
-for i in range(3):
-    p[0].data.mul_(1.5).add_(0.25)
-    ema.update(p)
-    trace.append(ema.shadow_params[0].double().tolist())
-res["ema"] = trace
-# optimiser + optimization_manager on CPU: warm-up lr, clip, one Adam step (losses.py:26-52)
-torch.manual_seed(0)
-w = [torch.nn.Parameter(torch.randn(5, 3)), torch.nn.Parameter(torch.randn(7))]
-opt = rlosses.get_optimizer(config, w)
-fn = rlosses.optimization_manager(config)
-steps = []
-g = torch.Generator().manual_seed(1)
-for step in (0, 10, 4999, 20000):
-    for q in w:
-        q.grad = torch.randn(q.shape, generator=g) * 3.0
-    fn(opt, w, step=step)
-    steps.append({"lr": opt.param_groups[0]["lr"], "w0": w[0].detach().double().flatten().tolist(), "w1": w[1].detach().double().tolist()})
-res["optim"] = {"steps": steps, "defaults": {k: (list(v) if isinstance(v, tuple) else v) for k, v in opt.defaults.items()
-                                              if k in ("lr", "betas", "eps", "weight_decay", "amsgrad")}}
-res["sigmas"] = [float(v) for v in ref["mutils"].get_sigmas(config)]
-# initial weights of a tiny network (the reference's own initialisers): per-tensor statistics
-config.data.image_size, config.model.nf, config.model.ch_mult = 16, 32, (1, 2)
-config.model.num_res_blocks, config.model.attn_resolutions = 1, (8,)
-torch.manual_seed(5)
-m = ref["mutils"].create_model(config)
-res["init"] = {k: {"std": float(v.double().std()) if v.numel() > 1 else 0.0, "absmax": float(v.abs().max()), "mean": float(v.double().mean()),
-                   "numel": v.numel(), "const": bool((v == v.flatten()[0]).all())}
-               for k, v in m.state_dict().items() if v.dtype.is_floating_point and k.split(".")[-1] not in ("sigmas", "mask", "coords")}
-json.dump(res, open(out, "w"))
-print("REF_DONE")
-'''
-
-
-def _have_reference():
-    return os.path.exists(os.path.join(ROOT, "baseline", "_ref", "lib", "diffusion", "sampling.py"))
+from helpers import GOLD
 
 
 @pytest.fixture(scope="module")
-def ref(tmp_path_factory):
-    if not _have_reference():
-        pytest.skip("baseline/_ref not staged (python baseline/install_reference.py)")
-    out = str(tmp_path_factory.mktemp("ref") / "ref.json")
-    r = subprocess.run([sys.executable, "-c", REF_SIDE, ROOT, out], capture_output=True, text=True, timeout=600,
-                       env=dict(os.environ, OMP_NUM_THREADS="4"))
-    assert r.returncode == 0 and "REF_DONE" in r.stdout, r.stdout + r.stderr
-    return json.load(open(out))
+def ref():
+    return json.load(lzma.open(os.path.join(GOLD, "reference_host.json.xz"), "rt"))
 
 
 def _flat(c, pre=""):

@@ -1,96 +1,25 @@
 """CPU: the host loop of the sampler -- every registered predictor / corrector pair, the partial (`cond_gen`) branch with the
 reference's (B,B,...) initial-broadcast quirk and `freeze_iters`, and `return_traj` -- is BITWISE equal to the REFERENCE's own
-`get_sampling_fn -> pc_sampler` (lib/diffusion/sampling.py:83-132,357-487, run from baseline/_ref in a subprocess) when both
-drive the same stub score model with the same seed. (On a CUDA tensor with the native network the configured
+`get_sampling_fn -> pc_sampler` (lib/diffusion/sampling.py:83-132,357-487; its outputs stored in
+tests/golden/reference_samplers.npz by oracle/make_host_golden.py) when both drive the stub score model of
+oracle/sampler_stub.py with the same seed. (On a CUDA tensor with the native network the configured
 ancestral + none pair takes the fused path instead; that path is pinned against reference goldens in tests/test_gpu_sampler.py.)"""
 import os
-import subprocess
-import sys
 
+import numpy as np
 import pytest
 import torch
 
-from helpers import ROOT
-
-STUB = r'''
-import torch
-class Stub(torch.nn.Module):
-    """Deterministic stand-in for model(x, labels): smooth, label-dependent, mixes neighbouring voxels."""
-    def __init__(self):
-        super().__init__()
-        self.w = torch.nn.Parameter(torch.tensor(0.37))
-    def forward(self, x, labels):
-        return torch.tanh(self.w * x + 1e-3 * labels.view(-1, 1, 1, 1, 1)) - 0.1 * x.roll(1, 2)
-
-def inputs(R, B):
-    g = torch.Generator().manual_seed(77)
-    mask = (torch.rand(1, 1, R, R, R, generator=g) < 0.7).float()
-    partial = torch.sign(torch.randn(1, 4, R, R, R, generator=g))
-    pmask = (torch.rand(1, 4, R, R, R, generator=g) < 0.5).float()
-    return mask, partial, pmask
-
-VARIANTS = [  # name, predictor, corrector, n_steps_each, probability_flow, partial, freeze_iters, return_traj, R, iters
-    ("ancestral", "ancestral_sampling", "none", 1, False, False, None, False, 8, 25),
-    ("em_langevin", "euler_maruyama", "langevin", 2, False, False, None, False, 8, 25),
-    ("rd_ald", "reverse_diffusion", "ald", 1, False, False, None, False, 8, 25),
-    ("rd_pflow", "reverse_diffusion", "none", 1, True, False, None, False, 8, 25),  # (EM + probability_flow raises in the reference: sampling.py:195)
-    ("none_langevin", "none", "langevin", 1, False, False, None, False, 8, 25),
-    ("partial", "ancestral_sampling", "none", 1, False, True, 10, False, 8, 25),
-    ("partial_all", "reverse_diffusion", "langevin", 1, False, True, None, False, 8, 12),
-    ("traj", "ancestral_sampling", "none", 1, False, False, None, True, 4, None),
-]
-'''
-
-REF_SIDE = STUB + r'''
-import sys
-root, out = sys.argv[1:3]
-sys.path.insert(0, root)
-from baseline import reference_arm
-ref, config = reference_arm.load("cpu")
-sampling, sde_lib = ref["sampling"], ref["sde_lib"]
-sde = sde_lib.VPSDE(beta_min=config.model.beta_min, beta_max=config.model.beta_max, N=config.model.num_scales)
-res = {}
-for name, pred, corr, nse, pflow, use_partial, freeze, traj, R, iters in VARIANTS:
-    B = 2
-    mask, partial, pmask = inputs(R, B)
-    config.sampling.method, config.sampling.predictor, config.sampling.corrector = "pc", pred, corr
-    config.sampling.n_steps_each, config.sampling.probability_flow, config.sampling.snr = nse, pflow, 0.16
-    fn = sampling.get_sampling_fn(config, sde, (B, 4, R, R, R), lambda x: x, 1e-3, grid_mask=mask, return_traj=traj)
-    real = sampling.tqdm.trange
-    if iters is not None:
-        sampling.tqdm.trange = lambda n, *a, **k: range(min(n, iters))
-    try:
-        torch.manual_seed(123)
-        kw = dict(partial=partial, partial_mask=pmask, partial_channel=0, freeze_iters=freeze) if use_partial else {}
-        o, nfe = fn(Stub(), **kw)
-    finally:
-        sampling.tqdm.trange = real
-    res[name] = ([t.clone() for t in o] if traj else o.clone(), nfe)
-torch.save(res, out)
-print("REF_DONE")
-'''
-
-
-def _have_reference():
-    return os.path.exists(os.path.join(ROOT, "baseline", "_ref", "lib", "diffusion", "sampling.py"))
+from helpers import GOLD
+from oracle.sampler_stub import VARIANTS, Stub, inputs
 
 
 @pytest.fixture(scope="module")
-def ref(tmp_path_factory):
-    if not _have_reference():
-        pytest.skip("baseline/_ref not staged (python baseline/install_reference.py)")
-    out = str(tmp_path_factory.mktemp("ref") / "samplers.pt")
-    r = subprocess.run([sys.executable, "-c", REF_SIDE, ROOT, out], capture_output=True, text=True, timeout=900,
-                       env=dict(os.environ, OMP_NUM_THREADS="4"))
-    assert r.returncode == 0 and "REF_DONE" in r.stdout, r.stdout + r.stderr
-    return torch.load(out, map_location="cpu", weights_only=False)
+def ref():
+    return np.load(os.path.join(GOLD, "reference_samplers.npz"))
 
 
-_ns = {}
-exec(STUB, _ns)
-
-
-@pytest.mark.parametrize("variant", _ns["VARIANTS"], ids=[v[0] for v in _ns["VARIANTS"]])
+@pytest.mark.parametrize("variant", VARIANTS, ids=[v[0] for v in VARIANTS])
 def test_host_sampler_loop_is_bitwise_the_reference(ref, variant):
     from configs import res64
     from meshdiffusion_b200.diffusion import sampling, sde_lib
@@ -102,13 +31,13 @@ def test_host_sampler_loop_is_bitwise_the_reference(ref, variant):
     if iters is not None:
         cfg.sampling.max_iters = iters
     B = 2
-    mask, partial, pmask = _ns["inputs"](R, B)
+    mask, partial, pmask = inputs(R, B)
     sde = sde_lib.VPSDE(beta_min=cfg.model.beta_min, beta_max=cfg.model.beta_max, N=cfg.model.num_scales, device="cpu")
     fn = sampling.get_sampling_fn(cfg, sde, (B, 4, R, R, R), lambda x: x, 1e-3, grid_mask=mask, return_traj=traj)
     torch.manual_seed(123)
     kw = dict(partial=partial, partial_mask=pmask, partial_channel=0, freeze_iters=freeze) if use_partial else {}
-    out, nfe = fn(_ns["Stub"](), **kw)
-    want, want_nfe = ref[name]
+    out, nfe = fn(Stub(), **kw)
+    want, want_nfe = torch.from_numpy(ref[name]), int(ref[name + "_nfe"])
     assert nfe == want_nfe
     if traj:
         assert len(out) == len(want) and len(out) > 0
