@@ -9,7 +9,10 @@ import ml_collections  # noqa: E402
 _DEFAULTS = {
     "training": dict(batch_size=64, n_iters=2400001, snapshot_freq=50000, log_freq=50, eval_freq=100,
                      snapshot_freq_for_preemption=5000, snapshot_sampling=True, likelihood_weighting=False,
-                     continuous=True, reduce_mean=False, iter_size=1, loss_type="l2", train_dir="PLACEHOLDER"),
+                     continuous=True, reduce_mean=False, iter_size=1, loss_type="l2", train_dir="PLACEHOLDER",
+                     # engine knob (not a reference key): training operand mode, 'bf16' or 'bf16x3' (split bf16, fp32-class
+                     # gradients at about a third of the tensor rate)
+                     compute_dtype="bf16"),
     "sampling": dict(n_steps_each=1, noise_removal=True, probability_flow=False, snr=0.075),
     "eval": dict(begin_ckpt=50, end_ckpt=96, batch_size=512, enable_sampling=True, num_samples=50000, enable_loss=True,
                  enable_bpd=False, bpd_dataset="test", ckpt_path="PLACEHOLDER", partial_dmtet_path="PLACEHOLDER",

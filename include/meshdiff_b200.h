@@ -39,7 +39,8 @@ typedef struct mdb_unet_config {
   int precision;           /* 0 = bf16 operands, 1 = tf32 operands, 2 = split bf16 ("bf16x3": every value is a (hi, lo)
                               bf16 pair and every product hi*hi + hi*lo + lo*hi -- fp32-class results, the mode that
                               meets the 1e-3 parity contract); fp32 accumulation in all three */
-  int training;            /* 1 = also build the backward plan (bf16 operands only) and keep what it needs */
+  int training;            /* 1 = also build the backward plan and keep what it needs; precision 0 (bf16) or 2 (bf16x3:
+                              split-bf16 activations, data and weight gradients for fp32-class gradients), not tf32 */
 } mdb_unet_config;
 
 int mdb_unet_create(const mdb_unet_config* cfg, mdb_unet** out);

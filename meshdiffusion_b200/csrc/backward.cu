@@ -1,4 +1,6 @@
-// Bandwidth-bound kernels of the training backward pass (bf16 activations, fp32 parameter gradients).
+// Bandwidth-bound kernels of the training backward pass (bf16 or split-bf16 activations, fp32 parameter gradients).
+// X3 (split bf16, gemm_host.h::kBF16X3): a tensor of logical row pitch ld stores [ld hi | ld lo] bf16 per voxel; the
+// kernels read hi + lo as one fp32 value and write what they compute back as a (hi, lo) pair.
 #include "backward.cuh"
 #include "gn_stats.cuh"
 #include <stdexcept>
@@ -25,6 +27,21 @@ __device__ __forceinline__ uint4 pack8(const float* x) {
 #pragma unroll
   for (int j = 0; j < 4; ++j) h[j] = __floats2bfloat162_rn(x[2 * j], x[2 * j + 1]);
   return t;
+}
+// X3: 8 channels as hi + lo, and back (lo = what the bf16 rounding of hi lost)
+__device__ __forceinline__ void unpack8x(const uint4& hi, const uint4& lo, float* x) {
+  float l[VEC];
+  unpack8(hi, x); unpack8(lo, l);
+#pragma unroll
+  for (int j = 0; j < VEC; ++j) x[j] += l[j];
+}
+__device__ __forceinline__ void pack8x(const float* x, uint4& hi, uint4& lo) {
+  float h[VEC], r[VEC];
+  hi = pack8(x);
+  unpack8(hi, h);
+#pragma unroll
+  for (int j = 0; j < VEC; ++j) r[j] = x[j] - h[j];
+  lo = pack8(r);
 }
 __device__ __forceinline__ float sigmoid_fast(float x) {
   float t;
@@ -93,8 +110,10 @@ __device__ __forceinline__ void gn_dy(const GnBwdArgs& a, const float* x, const 
 
 // Pass 1. Per element: h = 0.5*y straight from x (one FMA with folded constants), silu'(y) = t + 0.5*h*q with
 // t = (1+tanh h)/2, q = 1 - tanh^2 h; S2 is accumulated as sum(dy*x) and rebased to sum(dy*xhat) once per thread.
+template <bool X3>
 __global__ void __launch_bounds__(256, 2) gn_bwd_reduce_kernel(GnBwdArgs a, int cv, int k) {
-  constexpr int UNROLL = 4;
+  constexpr int UNROLL = X3 ? 2 : 4;  // X3: twice the bytes per voxel in flight, within the 128-register budget
+  constexpr long long PP = X3 ? 2 : 1;  // physical / logical row pitch
   __shared__ float red[256 * VEC * 2];
   const int C = a.C0 + a.C1;
   const int b = blockIdx.y;
@@ -112,28 +131,34 @@ __global__ void __launch_bounds__(256, 2) gn_bwd_reduce_kernel(GnBwdArgs a, int 
     }
   }
   const bool first = c < a.C0;
-  const char* src = first ? (const char*)a.x0 + ((long long)b * a.voxels * a.ld0 + c) * 2
-                          : (const char*)a.x1 + ((long long)b * a.voxels * a.ld1 + (c - a.C0)) * 2;
-  const long long src_stride = (first ? a.ld0 : a.ld1) * 2;
-  char* dsrc = const_cast<char*>((const char*)a.da) + ((long long)b * a.voxels * C + c) * 2;
-  const long long d_stride = (long long)C * 2;
+  const char* src = first ? (const char*)a.x0 + ((long long)b * a.voxels * a.ld0 * PP + c) * 2
+                          : (const char*)a.x1 + ((long long)b * a.voxels * a.ld1 * PP + (c - a.C0)) * 2;
+  const long long src_lo = (first ? a.ld0 : a.ld1) * 2;
+  const long long src_stride = src_lo * PP;
+  char* dsrc = const_cast<char*>((const char*)a.da) + ((long long)b * a.voxels * C * PP + c) * 2;
+  const long long d_lo = (long long)C * 2;
+  const long long d_stride = d_lo * PP;
   float s1[VEC], s2[VEC];
 #pragma unroll
   for (int j = 0; j < VEC; ++j) { s1[j] = 0.f; s2[j] = 0.f; }
   const long long step = (long long)gridDim.x * k;
   for (long long v0 = (long long)blockIdx.x * k + vl; v0 < a.voxels; v0 += step * UNROLL) {
-    uint4 rx[UNROLL], rd[UNROLL];
+    uint4 rx[UNROLL], rd[UNROLL], rxl[X3 ? UNROLL : 1], rdl[X3 ? UNROLL : 1];
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
       const long long v = v0 + u * step;
-      if (v < a.voxels) { rx[u] = __ldg((const uint4*)(src + v * src_stride)); rd[u] = *((const uint4*)(dsrc + v * d_stride)); }
+      if (v < a.voxels) {
+        rx[u] = __ldg((const uint4*)(src + v * src_stride)); rd[u] = *((const uint4*)(dsrc + v * d_stride));
+        if constexpr (X3) { rxl[u] = __ldg((const uint4*)(src + v * src_stride + src_lo)); rdl[u] = *((const uint4*)(dsrc + v * d_stride + d_lo)); }
+      }
     }
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
       const long long v = v0 + u * step;
       if (v >= a.voxels) continue;
       float x[VEC], dy[VEC];
-      unpack8(rx[u], x); unpack8(rd[u], dy);
+      if constexpr (X3) { unpack8x(rx[u], rxl[u], x); unpack8x(rd[u], rdl[u], dy); }
+      else { unpack8(rx[u], x); unpack8(rd[u], dy); }
       if (a.drop_thresh > 0) {
         const unsigned long long e4 = (unsigned long long)((((long long)b * a.voxels + v) * C + c) >> 2);
         const unsigned long long h0 = drop_hash64(a.seed, e4), h1 = drop_hash64(a.seed, e4 + 1);
@@ -157,7 +182,8 @@ __global__ void __launch_bounds__(256, 2) gn_bwd_reduce_kernel(GnBwdArgs a, int 
 #pragma unroll
       for (int j = 0; j < VEC; ++j) { s1[j] += dy[j]; s2[j] = fmaf(dy[j], x[j], s2[j]); }
       // dy replaces da in place: pass 2 then needs neither the activation derivative nor the dropout hash again
-      *((uint4*)(dsrc + v * d_stride)) = pack8(dy);
+      if constexpr (X3) pack8x(dy, *((uint4*)(dsrc + v * d_stride)), *((uint4*)(dsrc + v * d_stride + d_lo)));
+      else *((uint4*)(dsrc + v * d_stride)) = pack8(dy);
     }
   }
   {
@@ -208,7 +234,8 @@ void launch_gn_bwd_reduce(const GnBwdArgs& a, int B, cudaStream_t s) {
   gn_launch_shape(a, cv, k);
   const int C = a.C0 + a.C1;
   const int gx = blocks_x(a.voxels, k, B, 296);
-  gn_bwd_reduce_kernel<<<dim3(gx, B), cv * k, 0, s>>>(a, cv, k);
+  if (a.x3) gn_bwd_reduce_kernel<true><<<dim3(gx, B), cv * k, 0, s>>>(a, cv, k);
+  else gn_bwd_reduce_kernel<false><<<dim3(gx, B), cv * k, 0, s>>>(a, cv, k);
   MDB_LAUNCH_CHECK();
   gn_bwd_sums_kernel<<<(B * C + 255) / 256, 256, 0, s>>>(a.part, a.sums, gx, B * C);
   MDB_LAUNCH_CHECK();
@@ -217,7 +244,7 @@ void launch_gn_bwd_reduce(const GnBwdArgs& a, int B, cudaStream_t s) {
 }
 
 constexpr int kApplyDepth = 4;
-constexpr int kApplySmem = kApplyDepth * 4 * 256 * 16;  // 64 KB
+constexpr int kApplySmem = kApplyDepth * 4 * 256 * 16;  // 64 KB (X3: twice the streams at half the depth)
 __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
 }
@@ -226,8 +253,11 @@ template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 // NADD = number of addend streams (0, 1, 2): absent streams cost no instructions (GroupNorm_1 layers have none)
-template <int NADD>
-__global__ void __launch_bounds__(256, 3) gn_bwd_apply_kernel(GnBwdArgs a, int cv, int k) {
+template <int NADD, bool X3>
+__global__ void __launch_bounds__(256, X3 ? 2 : 3) gn_bwd_apply_kernel(GnBwdArgs a, int cv, int k) {
+  constexpr int DEPTH = X3 ? kApplyDepth / 2 : kApplyDepth;
+  constexpr int NS = X3 ? 8 : 4;        // ring slots per stage: (x, dy, add0, add1), X3: hi and lo of each
+  constexpr long long PP = X3 ? 2 : 1;  // physical / logical row pitch
   __shared__ float red[256 * VEC];
   const int C = a.C0 + a.C1;
   const int b = blockIdx.y;
@@ -262,14 +292,16 @@ __global__ void __launch_bounds__(256, 3) gn_bwd_apply_kernel(GnBwdArgs a, int c
     }
   }
   const bool first = c < a.C0;
-  const char* src = first ? (const char*)a.x0 + ((long long)b * a.voxels * a.ld0 + c) * 2
-                          : (const char*)a.x1 + ((long long)b * a.voxels * a.ld1 + (c - a.C0)) * 2;
-  const long long src_stride = (first ? a.ld0 : a.ld1) * 2;
-  const char* dsrc = (const char*)a.da + ((long long)b * a.voxels * C + c) * 2;
-  const long long d_stride = (long long)C * 2;
-  char* dst = (char*)a.dx + ((long long)b * a.voxels * C + c) * 2;
-  const char* p0 = NADD >= 1 ? (const char*)a.add0 + ((long long)b * a.voxels * a.add0_ld + c) * 2 : nullptr;
-  const char* p1 = NADD >= 2 ? (const char*)a.add1 + ((long long)b * a.voxels * a.add1_ld + c) * 2 : nullptr;
+  const char* src = first ? (const char*)a.x0 + ((long long)b * a.voxels * a.ld0 * PP + c) * 2
+                          : (const char*)a.x1 + ((long long)b * a.voxels * a.ld1 * PP + (c - a.C0)) * 2;
+  const long long src_lo = (first ? a.ld0 : a.ld1) * 2;
+  const long long src_stride = src_lo * PP;
+  const char* dsrc = (const char*)a.da + ((long long)b * a.voxels * C * PP + c) * 2;
+  const long long d_lo = (long long)C * 2;
+  const long long d_stride = d_lo * PP;
+  char* dst = (char*)a.dx + ((long long)b * a.voxels * C * PP + c) * 2;
+  const char* p0 = NADD >= 1 ? (const char*)a.add0 + ((long long)b * a.voxels * a.add0_ld * PP + c) * 2 : nullptr;
+  const char* p1 = NADD >= 2 ? (const char*)a.add1 + ((long long)b * a.voxels * a.add1_ld * PP + c) * 2 : nullptr;
   float cs[VEC];
 #pragma unroll
   for (int j = 0; j < VEC; ++j) cs[j] = 0.f;
@@ -278,47 +310,57 @@ __global__ void __launch_bounds__(256, 3) gn_bwd_apply_kernel(GnBwdArgs a, int c
   // ring (no barriers: a thread only ever reads what it copied itself). The register-staged version of this kernel was
   // latency-bound at ~3.7 TB/s (ncu: 7 warps stalled on long-scoreboard per issue, 25-37 % occupancy); with 3 blocks/SM
   // and 4 stages there are up to 190 KB of requests outstanding per SM.
-  extern __shared__ uint4 ring[];  // [kApplyDepth][4 streams][256 threads]
-  auto slot = [&](int stage, int stream) { return ring + ((stage * 4 + stream) * 256 + threadIdx.x); };
+  extern __shared__ uint4 ring[];  // [DEPTH][NS streams][256 threads]
+  auto slot = [&](int stage, int stream) { return ring + ((stage * NS + stream) * 256 + threadIdx.x); };
   auto issue = [&](long long vv, int stage) {
     if (vv < a.voxels) {
       cp_async16(slot(stage, 0), src + vv * src_stride);
       cp_async16(slot(stage, 1), dsrc + vv * d_stride);
-      if (NADD >= 1) cp_async16(slot(stage, 2), p0 + vv * a.add0_ld * 2);
-      if (NADD >= 2) cp_async16(slot(stage, 3), p1 + vv * a.add1_ld * 2);
+      if (NADD >= 1) cp_async16(slot(stage, 2), p0 + vv * a.add0_ld * 2 * PP);
+      if (NADD >= 2) cp_async16(slot(stage, 3), p1 + vv * a.add1_ld * 2 * PP);
+      if constexpr (X3) {
+        cp_async16(slot(stage, 4), src + vv * src_stride + src_lo);
+        cp_async16(slot(stage, 5), dsrc + vv * d_stride + d_lo);
+        if (NADD >= 1) cp_async16(slot(stage, 6), p0 + vv * a.add0_ld * 2 * PP + a.add0_ld * 2);
+        if (NADD >= 2) cp_async16(slot(stage, 7), p1 + vv * a.add1_ld * 2 * PP + a.add1_ld * 2);
+      }
     }
     cp_async_commit();
   };
+  auto get = [&](int stage, int stream, float* x) {
+    if constexpr (X3) unpack8x(*slot(stage, stream), *slot(stage, stream + 4), x);
+    else unpack8(*slot(stage, stream), x);
+  };
   long long v = (long long)blockIdx.x * k + vl;
 #pragma unroll
-  for (int d = 0; d < kApplyDepth - 1; ++d) issue(v + d * step, d);
+  for (int d = 0; d < DEPTH - 1; ++d) issue(v + d * step, d);
   int stage = 0;
   for (; v < a.voxels; v += step) {
-    int nst = stage + kApplyDepth - 1;
-    if (nst >= kApplyDepth) nst -= kApplyDepth;
-    issue(v + (long long)(kApplyDepth - 1) * step, nst);
-    cp_async_wait<kApplyDepth - 1>();
-    const uint4 cx = *slot(stage, 0), cd = *slot(stage, 1);
+    int nst = stage + DEPTH - 1;
+    if (nst >= DEPTH) nst -= DEPTH;
+    issue(v + (long long)(DEPTH - 1) * step, nst);
+    cp_async_wait<DEPTH - 1>();
     float x[VEC], dy[VEC], o[VEC];
-    unpack8(cx, x); unpack8(cd, dy);
+    get(stage, 0, x); get(stage, 1, dy);
 #pragma unroll
     for (int j = 0; j < VEC; ++j) o[j] = fmaf(-x[j], k1[j], fmaf(c1[j], dy[j], -k0[j]));
     if (NADD >= 1) {
       float e[VEC];
-      unpack8(*slot(stage, 2), e);
+      get(stage, 2, e);
 #pragma unroll
       for (int j = 0; j < VEC; ++j) o[j] += e[j];
     }
     if (NADD >= 2) {
       float e[VEC];
-      unpack8(*slot(stage, 3), e);
+      get(stage, 3, e);
 #pragma unroll
       for (int j = 0; j < VEC; ++j) o[j] += e[j];
     }
 #pragma unroll
     for (int j = 0; j < VEC; ++j) cs[j] += o[j];
-    *((uint4*)(dst + v * d_stride)) = pack8(o);
-    if (++stage == kApplyDepth) stage = 0;
+    if constexpr (X3) pack8x(o, *((uint4*)(dst + v * d_stride)), *((uint4*)(dst + v * d_stride + d_lo)));
+    else *((uint4*)(dst + v * d_stride)) = pack8(o);
+    if (++stage == DEPTH) stage = 0;
   }
   cp_async_wait<0>();
   if (a.cs_part) {  // per-(sample, channel) column sums of dx for the bias / time-embedding gradients downstream
@@ -353,17 +395,26 @@ void launch_gn_bwd_apply(const GnBwdArgs& a, int B, cudaStream_t s) {
   cudaGetDevice(&dev);
   bool& configured = configured_dev[dev < 64 ? dev : 63];
   if (!configured || dev >= 63) {
-    cudaFuncSetAttribute(gn_bwd_apply_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, kApplySmem);
-    cudaFuncSetAttribute(gn_bwd_apply_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, kApplySmem);
-    cudaFuncSetAttribute(gn_bwd_apply_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, kApplySmem);
+    cudaFuncSetAttribute(gn_bwd_apply_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kApplySmem);
+    cudaFuncSetAttribute(gn_bwd_apply_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kApplySmem);
+    cudaFuncSetAttribute(gn_bwd_apply_kernel<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kApplySmem);
+    cudaFuncSetAttribute(gn_bwd_apply_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kApplySmem);
+    cudaFuncSetAttribute(gn_bwd_apply_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kApplySmem);
+    cudaFuncSetAttribute(gn_bwd_apply_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kApplySmem);
     configured = true;
   }
   GnBwdArgs q = a;
   if (!q.add0 && q.add1) { q.add0 = q.add1; q.add0_ld = q.add1_ld; q.add1 = nullptr; }  // streams are filled front to back
   const dim3 grid((unsigned)gx, B);
-  if (q.add1) gn_bwd_apply_kernel<2><<<grid, cv * k, kApplySmem, s>>>(q, cv, k);
-  else if (q.add0) gn_bwd_apply_kernel<1><<<grid, cv * k, kApplySmem, s>>>(q, cv, k);
-  else gn_bwd_apply_kernel<0><<<grid, cv * k, kApplySmem, s>>>(q, cv, k);
+  if (q.x3) {
+    if (q.add1) gn_bwd_apply_kernel<2, true><<<grid, cv * k, kApplySmem, s>>>(q, cv, k);
+    else if (q.add0) gn_bwd_apply_kernel<1, true><<<grid, cv * k, kApplySmem, s>>>(q, cv, k);
+    else gn_bwd_apply_kernel<0, true><<<grid, cv * k, kApplySmem, s>>>(q, cv, k);
+  } else {
+    if (q.add1) gn_bwd_apply_kernel<2, false><<<grid, cv * k, kApplySmem, s>>>(q, cv, k);
+    else if (q.add0) gn_bwd_apply_kernel<1, false><<<grid, cv * k, kApplySmem, s>>>(q, cv, k);
+    else gn_bwd_apply_kernel<0, false><<<grid, cv * k, kApplySmem, s>>>(q, cv, k);
+  }
   MDB_LAUNCH_CHECK();
   if (a.cs_part) {
     cs_final_kernel<<<(B * C + 255) / 256, 256, 0, s>>>(a.cs_part, a.cs_per, gx, B * C);
@@ -427,29 +478,36 @@ void launch_gnb_tile_reduce(const GnBwdArgs& a, const float* tile_part, int T, i
 }
 
 // ------------------------------------------------------------------ column sums (bias / time-embedding gradients)
+template <bool X3>
 __global__ void __launch_bounds__(256) colsum_kernel(ColsumArgs a, int cv, int k) {
   constexpr int UNROLL = 4;
+  constexpr long long PP = X3 ? 2 : 1;
   __shared__ float red[256 * VEC];
   const int b = blockIdx.y;
   const int cvi = threadIdx.x % cv, vl = threadIdx.x / cv;
   const int c = cvi * VEC;
-  const char* src = (const char*)a.t + ((long long)b * a.voxels * a.ld + c) * 2;
+  const char* src = (const char*)a.t + ((long long)b * a.voxels * a.ld * PP + c) * 2;
   float s1[VEC];
 #pragma unroll
   for (int j = 0; j < VEC; ++j) s1[j] = 0.f;
   const long long step = (long long)gridDim.x * k;
   for (long long v0 = (long long)blockIdx.x * k + vl; v0 < a.voxels; v0 += step * UNROLL) {
-    uint4 r[UNROLL];
+    uint4 r[UNROLL], rl[X3 ? UNROLL : 1];
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
       const long long v = v0 + u * step;
       r[u] = make_uint4(0, 0, 0, 0);
-      if (v < a.voxels) r[u] = __ldg((const uint4*)(src + v * a.ld * 2));
+      if constexpr (X3) rl[u] = make_uint4(0, 0, 0, 0);
+      if (v < a.voxels) {
+        r[u] = __ldg((const uint4*)(src + v * a.ld * 2 * PP));
+        if constexpr (X3) rl[u] = __ldg((const uint4*)(src + v * a.ld * 2 * PP + a.ld * 2));
+      }
     }
 #pragma unroll
     for (int u = 0; u < UNROLL; ++u) {
       float x[VEC];
-      unpack8(r[u], x);
+      if constexpr (X3) unpack8x(r[u], rl[u], x);
+      else unpack8(r[u], x);
 #pragma unroll
       for (int j = 0; j < VEC; ++j) s1[j] += x[j];
     }
@@ -506,7 +564,8 @@ void launch_colsum(const ColsumArgs& a, int B, cudaStream_t s) {
   if (cv < 1 || cv > 256 || a.C % VEC != 0) throw std::runtime_error("mdb: unsupported channel count in colsum");
   const int k = 256 / cv;
   const int gx = blocks_x(a.voxels, k, B, 592);
-  colsum_kernel<<<dim3(gx, B), cv * k, 0, s>>>(a, cv, k);
+  if (a.x3) colsum_kernel<true><<<dim3(gx, B), cv * k, 0, s>>>(a, cv, k);
+  else colsum_kernel<false><<<dim3(gx, B), cv * k, 0, s>>>(a, cv, k);
   MDB_LAUNCH_CHECK();
   colsum_final_kernel<<<(a.C + 31) / 32, dim3(32, 8), 0, s>>>(a, gx, B);
   MDB_LAUNCH_CHECK();
@@ -541,7 +600,10 @@ void launch_zero_stuff2x(const void* dy, void* z, int B, int R, int C, cudaStrea
   MDB_LAUNCH_CHECK();
 }
 
+// X3: rows of cv hi vectors then cv lo vectors
+template <bool X3>
 __global__ void downsum2x_kernel(const uint4* __restrict__ dup, uint4* __restrict__ dx, int B, int R, int cv) {
+  constexpr int PP = X3 ? 2 : 1;
   const int R2 = 2 * R;
   const long long total = (long long)B * R * R * R * cv;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
@@ -557,37 +619,53 @@ __global__ void downsum2x_kernel(const uint4* __restrict__ dup, uint4* __restric
       for (int dyy = 0; dyy < 2; ++dyy)
         for (int dxx = 0; dxx < 2; ++dxx) {
           float t[VEC];
-          unpack8(__ldg(dup + ((((long long)r * R2 + 2 * zo + dz) * R2 + 2 * yo + dyy) * R2 + 2 * xo + dxx) * cv + c), t);
+          const uint4* sp = dup + ((((long long)r * R2 + 2 * zo + dz) * R2 + 2 * yo + dyy) * R2 + 2 * xo + dxx) * cv * PP + c;
+          if constexpr (X3) unpack8x(__ldg(sp), __ldg(sp + cv), t);
+          else unpack8(__ldg(sp), t);
 #pragma unroll
           for (int j = 0; j < VEC; ++j) acc[j] += t[j];
         }
-    dx[i] = pack8(acc);
+    if constexpr (X3) {
+      uint4* dp = dx + (i - c) * PP + c;
+      pack8x(acc, dp[0], dp[cv]);
+    } else {
+      dx[i] = pack8(acc);
+    }
   }
 }
-void launch_downsum2x(const void* dup, void* dx, int B, int R, int C, cudaStream_t s) {
+void launch_downsum2x(const void* dup, void* dx, int B, int R, int C, int x3, cudaStream_t s) {
   const int cv = C / VEC;
   const long long total = (long long)B * R * R * R * cv;
-  downsum2x_kernel<<<grid_for(total, 256), 256, 0, s>>>((const uint4*)dup, (uint4*)dx, B, R, cv);
+  if (x3) downsum2x_kernel<true><<<grid_for(total, 256), 256, 0, s>>>((const uint4*)dup, (uint4*)dx, B, R, cv);
+  else downsum2x_kernel<false><<<grid_for(total, 256), 256, 0, s>>>((const uint4*)dup, (uint4*)dx, B, R, cv);
   MDB_LAUNCH_CHECK();
 }
 
-__global__ void batch_sum_kernel(const uint4* __restrict__ t, uint4* __restrict__ out, int B, long long n) {
+// n = logical vectors per sample; X3: rows of cv hi vectors then cv lo vectors
+template <bool X3>
+__global__ void batch_sum_kernel(const uint4* __restrict__ t, uint4* __restrict__ out, int B, long long n, int cv) {
+  constexpr int PP = X3 ? 2 : 1;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const long long pi = X3 ? (i / cv) * 2 * cv + i % cv : i;  // physical index of the (hi) vector
     float acc[VEC];
 #pragma unroll
     for (int j = 0; j < VEC; ++j) acc[j] = 0.f;
     for (int b = 0; b < B; ++b) {
       float x[VEC];
-      unpack8(__ldg(t + (long long)b * n + i), x);
+      const uint4* sp = t + (long long)b * n * PP + pi;
+      if constexpr (X3) unpack8x(__ldg(sp), __ldg(sp + cv), x);
+      else unpack8(__ldg(sp), x);
 #pragma unroll
       for (int j = 0; j < VEC; ++j) acc[j] += x[j];
     }
-    out[i] = pack8(acc);
+    if constexpr (X3) pack8x(acc, out[pi], out[pi + cv]);
+    else out[i] = pack8(acc);
   }
 }
-void launch_batch_sum(const void* t, void* out, int B, long long VC, cudaStream_t s) {
+void launch_batch_sum(const void* t, void* out, int B, long long VC, int C, int x3, cudaStream_t s) {
   const long long n = VC / VEC;
-  batch_sum_kernel<<<grid_for(n, 256), 256, 0, s>>>((const uint4*)t, (uint4*)out, B, n);
+  if (x3) batch_sum_kernel<true><<<grid_for(n, 256), 256, 0, s>>>((const uint4*)t, (uint4*)out, B, n, C / VEC);
+  else batch_sum_kernel<false><<<grid_for(n, 256), 256, 0, s>>>((const uint4*)t, (uint4*)out, B, n, C / VEC);
   MDB_LAUNCH_CHECK();
 }
 
@@ -614,6 +692,7 @@ void launch_rowsum_nc(const float* t, float* out, int B, int C, long long V, int
 }
 
 // ------------------------------------------------------------------ attention softmax backward (layers.py:604)
+template <bool X3>  // X3: P and dS rows are [L hi | L lo] bf16 (the same bytes as L fp32 slots)
 __global__ void __launch_bounds__(256) softmax_bwd_rows_kernel(const float* __restrict__ P, float* __restrict__ dP, long long rows, int L) {
   __shared__ float red[8];
   for (long long row = blockIdx.x; row < rows; row += gridDim.x) {
@@ -624,7 +703,7 @@ __global__ void __launch_bounds__(256) softmax_bwd_rows_kernel(const float* __re
 #pragma unroll
     for (int j = 0; j < 16; ++j) {
       const int i = threadIdx.x + j * 256;
-      pv[j] = i < L ? __bfloat162float(p[i]) : 0.f;
+      pv[j] = i < L ? __bfloat162float(p[i]) + (X3 ? __bfloat162float(p[L + i]) : 0.f) : 0.f;
       dv[j] = i < L ? d[i] : 0.f;
       dot = fmaf(pv[j], dv[j], dot);
     }
@@ -637,14 +716,20 @@ __global__ void __launch_bounds__(256) softmax_bwd_rows_kernel(const float* __re
 #pragma unroll
     for (int j = 0; j < 16; ++j) {
       const int i = threadIdx.x + j * 256;
-      if (i < L) reinterpret_cast<__nv_bfloat16*>(d)[i] = __float2bfloat16(pv[j] * (dv[j] - dot));
+      if (i < L) {
+        const float ds = pv[j] * (dv[j] - dot);
+        const __nv_bfloat16 hb = __float2bfloat16(ds);
+        reinterpret_cast<__nv_bfloat16*>(d)[i] = hb;
+        if (X3) reinterpret_cast<__nv_bfloat16*>(d)[L + i] = __float2bfloat16(ds - __bfloat162float(hb));
+      }
     }
   }
 }
-void launch_softmax_bwd_rows(const float* P, float* dP, long long rows, int L, cudaStream_t s) {
+void launch_softmax_bwd_rows(const float* P, float* dP, long long rows, int L, int x3, cudaStream_t s) {
   if (L > 16 * 256) throw std::runtime_error("mdb: softmax row too long");
   const int grid = (int)(rows < 148LL * 16 ? rows : 148LL * 16);
-  softmax_bwd_rows_kernel<<<grid, 256, 0, s>>>(P, dP, rows, L);
+  if (x3) softmax_bwd_rows_kernel<true><<<grid, 256, 0, s>>>(P, dP, rows, L);
+  else softmax_bwd_rows_kernel<false><<<grid, 256, 0, s>>>(P, dP, rows, L);
   MDB_LAUNCH_CHECK();
 }
 

@@ -39,6 +39,8 @@ struct GnBwdArgs {
   const void* add1; long long add1_ld;
   // optional by-product of pass 2: cs_per[b][c] = sum_v dx[b][v][c] (cs_part: [rows][C] block partials)
   float* cs_part; float* cs_per;
+  // 1: x0, x1, da, dx, add0, add1 are split-bf16 tensors ((hi, lo) rows, gemm_host.h::kBF16X3; pitches stay logical)
+  int x3;
 };
 void launch_gn_bwd_reduce(const GnBwdArgs& a, int B, cudaStream_t s);  // part -> sums -> dgamma/dbeta
 void launch_gn_bwd_apply(const GnBwdArgs& a, int B, cudaStream_t s);
@@ -58,22 +60,24 @@ struct ColsumArgs {
   float* per; long long per_ld;
   float* total0; float* total1; float* total2; int accumulate;
   const float* from_per; long long from_ld;  // per-sample sums already computed by the producing kernel ([B][from_ld])
+  int x3;                     // t is a split-bf16 tensor ((hi, lo) rows of logical pitch ld)
 };
 void launch_colsum(const ColsumArgs& a, int B, cudaStream_t s);
 
 // Downsample backward helper: z[b][2i+1 (each axis)][c] = dy[b][i][c], zero elsewhere (z has twice the extents).
+// Moves whole rows: a split-bf16 tensor is passed as 2C bf16 channels.
 void launch_zero_stuff2x(const void* dy, void* z, int B, int R, int C, cudaStream_t s);
-// Upsample backward: dx[b][i][c] = sum over the 2x2x2 block of d_up (R = extents of dx).
-void launch_downsum2x(const void* dup, void* dx, int B, int R, int C, cudaStream_t s);
-// out[v][c] = sum_b t[b][v][c]  (bf16)
-void launch_batch_sum(const void* t, void* out, int B, long long VC, cudaStream_t s);
+// Upsample backward: dx[b][i][c] = sum over the 2x2x2 block of d_up (R = extents of dx). x3: split-bf16 rows.
+void launch_downsum2x(const void* dup, void* dx, int B, int R, int C, int x3, cudaStream_t s);
+// out[v][c] = sum_b t[b][v][c]  (bf16, VC = voxels * C; x3: split-bf16 rows of C channels)
+void launch_batch_sum(const void* t, void* out, int B, long long VC, int C, int x3, cudaStream_t s);
 // out[c] (+)= sum_{b,v} t[b][c][v]  (fp32 NCDHW, e.g. the head bias gradient)
 void launch_rowsum_nc(const float* t, float* out, int B, int C, long long V, int accumulate, cudaStream_t s);
 
 // Attention softmax backward, in place: row r holds dP (fp32, L values); P holds the probabilities written by the
 // forward softmax (bf16 at the start of rows of L fp32 slots). Writes dS = P*(dP - sum(P*dP)) as bf16 at the start of
-// each dP row (same convention as the forward).
-void launch_softmax_bwd_rows(const float* P, float* dP, long long rows, int L, cudaStream_t s);
+// each dP row (same convention as the forward). x3: P and dS as [L hi | L lo] bf16 in the row's L fp32 slots.
+void launch_softmax_bwd_rows(const float* P, float* dP, long long rows, int L, int x3, cudaStream_t s);
 
 // dW[n][k] (+)= sum_b dy[b][n] x[b][k];  db[n] (+)= sum_b dy[b][n]      (fp32, small)
 void launch_outer_sum(const float* dy, long long dy_ld, const float* x, long long x_ld, float* dW, float* db, int B, int N, int K,

@@ -176,7 +176,7 @@ __global__ void __launch_bounds__(256, MODE == 1 ? 4 : 3) norm_act_kernel(NormAc
         if (a.silu) y = MODE == 0 ? silu_fast(y) : silu_f(y);
         x[j] = y;
       }
-      if (MODE == 0 && a.drop_thresh > 0) {
+      if (!TF32 && a.drop_thresh > 0) {  // (training plans: bf16 and split bf16; same element index in both)
         const unsigned long long e4 = (unsigned long long)((((long long)b * a.voxels + v) * C + c) >> 2);
         const unsigned long long h0 = drop_hash64(a.seed, e4), h1 = drop_hash64(a.seed, e4 + 1);
 #pragma unroll

@@ -333,14 +333,18 @@ void GemmOp::set_residual(const void* res, long long ldr, long long batch_stride
 
 void GemmOp::set_gn_backward(const void* x0, long long ld0, int c0, const void* x1, long long ld1, const void* consts, int silu,
                              float* part) {
-  if (prec != kBF16 || p.out_fp32 || p.ocs != 1) throw std::runtime_error("mdb: the GroupNorm-backward epilogue is built for bf16 NDHWC outputs");
+  if (prec == kTF32 || p.out_fp32 || p.ocs != 1) throw std::runtime_error("mdb: the GroupNorm-backward epilogue is built for bf16 / bf16x3 NDHWC outputs");
   if (p.N % 32 != 0 || (x1 && c0 % 32 != 0)) throw std::runtime_error("mdb: GroupNorm-backward epilogue needs 32-channel aligned sources");
   if (splits > 1) throw std::runtime_error("mdb: GroupNorm-backward epilogue cannot be combined with split-K");
   gnb = true;
+  // X3: the GroupNorm inputs are (hi, lo) rows -- physical pitches twice the logical ones, lo parts one logical row behind
+  const long long pp = parts(prec);
   p.res = x0; p.res_fp32 = 0; p.batch_fastest = 0;
-  p.rsx = ld0; p.rsy = ld0 * p.X; p.rsz = ld0 * p.X * p.Y; p.rsb = ld0 * p.X * p.Y * p.Z;
+  p.rsx = pp * ld0; p.rsy = p.rsx * p.X; p.rsz = p.rsy * p.Y; p.rsb = p.rsz * p.Z;
   p.res1 = x1; p.res_c0 = x1 ? c0 : p.N;
-  p.r1sx = ld1; p.r1sy = ld1 * p.X; p.r1sz = ld1 * p.X * p.Y; p.r1sb = ld1 * p.X * p.Y * p.Z;
+  p.r1sx = pp * ld1; p.r1sy = p.r1sx * p.X; p.r1sz = p.r1sy * p.Y; p.r1sb = p.r1sz * p.Z;
+  p.res_lo_off = prec == kBF16X3 ? ld0 : 0;
+  p.res1_lo_off = prec == kBF16X3 ? ld1 : 0;
   p.gnb_c = reinterpret_cast<const float4*>(consts);
   p.gnb_silu = silu;
   p.gnb_part = part;
@@ -589,9 +593,21 @@ void GemmOp::launch(cudaStream_t stream, int B, void* out_override) const {
   if (out_override) p.out = out_override;
   const int tiles_m = p.tx * p.ty * p.tz * p.tb;
   const bool tf = prec == kTF32;
+  const bool x3 = prec == kBF16X3;
   if (gnb) {
-    if (tf || p.splits > 1) throw std::runtime_error("mdb: GroupNorm-backward epilogue: bf16, no split-K");
+    if (tf || p.splits > 1) throw std::runtime_error("mdb: GroupNorm-backward epilogue: bf16 / bf16x3, no split-K");
     p.gnb_drop_thresh = rt_drop_thresh; p.gnb_drop_scale = rt_drop_scale; p.gnb_seed = rt_seed;
+    if (x3) {  // (m2 is never chosen for X3)
+      if (pair) {
+        const int pairs = sm_count() / 2, work = (tiles_m + 1) / 2 * p.n_tiles_n;
+        launch_impl<128, false, true, true, true>(p, 2 * (work < pairs ? work : pairs), stream);
+      } else {
+        const int total = tiles_m * p.n_tiles_n;
+        const int grid = total < sm_count() ? total : sm_count();
+        if (block_n == 32) launch_impl<32, false, false, true, true>(p, grid, stream); else launch_impl<128, false, false, true, true>(p, grid, stream);
+      }
+      return;
+    }
     if (pair) {
       const int work = (m2 ? (tiles_m + 3) / 4 : (tiles_m + 1) / 2) * p.n_tiles_n;
       const int pairs = sm_count() / 2;
@@ -604,7 +620,6 @@ void GemmOp::launch(cudaStream_t stream, int B, void* out_override) const {
     }
     return;
   }
-  const bool x3 = prec == kBF16X3;
   if (pair) {
     const int work = (m2 ? (tiles_m + 3) / 4 : (tiles_m + 1) / 2) * p.n_tiles_n;
     const int pairs = sm_count() / 2;

@@ -88,7 +88,8 @@ struct GemmParams {
   int b_explicit_k;    // B tile K coordinates come from LoadEntry::wc0 instead of the running k column
   int n_stages, stage_bytes;  // shared-memory operand ring: as many stages as fit next to the epilogue scratch
   // X3 (split bf16) epilogue: the lo parts of the output / residual rows sit this many elements behind the hi parts
-  long long out_lo_off, res_lo_off;
+  // (res1_lo_off: the second GroupNorm-backward source)
+  long long out_lo_off, res_lo_off, res1_lo_off;
   // epilogue
   void* out;
   long long osx, osy, osz, osb;  // output element strides per voxel axis
@@ -580,6 +581,11 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_tc_kernel(const __grid_c
           const uint4* rp = reinterpret_cast<const uint4*>(base + off);
 #pragma unroll
           for (int i = 0; i < 4; ++i) rbuf[i] = __ldg(rp + i);
+          if constexpr (X3) {
+            const uint4* rl = reinterpret_cast<const uint4*>(base + off + (second ? p.res1_lo_off : p.res_lo_off));
+#pragma unroll
+            for (int i = 0; i < 4; ++i) rbuf[4 + i] = __ldg(rl + i);
+          }
           return;
         }
         if (TF32 || p.res_fp32) {
@@ -659,7 +665,8 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_tc_kernel(const __grid_c
             for (int i = 0; i < 32; ++i) {
               const float4 kc = __ldg(cc + i);
               const __nv_bfloat16 xb = reinterpret_cast<const __nv_bfloat16*>(rbuf)[i];
-              const float xv = __bfloat162float(xb);
+              float xv = __bfloat162float(xb);
+              if constexpr (X3) xv += __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(rbuf + 4)[i]);
               float d = v[i];
               if (p.gnb_drop_thresh > 0) {
                 const unsigned r16 = (unsigned)((hsh[i >> 2] >> (16 * (i & 3))) & 0xFFFFu);

@@ -590,7 +590,7 @@ UNet::UNet(const UNetConfig& cfg, bool dry_only) : cfg_(cfg), prec_(precision_fr
   if (cfg_.nf % 32 != 0) throw std::runtime_error("mdb: nf must be a multiple of 32 (GroupNorm(32))");
   train_ = cfg_.training != 0;
   if (const char* e = getenv("MDB_GRAPH_MAX_BATCH")) graph_max_batch_ = atoi(e);  // 0 disables graph replay
-  if (train_ && prec_ != kBF16) throw std::runtime_error("mdb: the training plan is built for bf16 operands");
+  if (train_ && prec_ == kTF32) throw std::runtime_error("mdb: the training plan is built for bf16 or bf16x3 operands");
   dry_ = true;
   build();
   // allocate everything the dry run sized

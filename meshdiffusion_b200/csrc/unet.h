@@ -27,8 +27,8 @@ struct UNetConfig {
   int stem_ksize = 3;   // 3 (res64) or 5 (res128)
   int use_pos_bias = 1; // ddpm_res64.py:148 adds pos_layer(coords*0) == its bias; res128 does not
   int max_batch = 1;
-  int precision = 0;    // 0 = bf16 operands, 1 = tf32 operands (fp32 accumulate in TMEM either way)
-  int training = 0;     // 1: keep the activations backward needs and build the backward plan (bf16 only)
+  int precision = 0;    // 0 = bf16 operands, 1 = tf32 operands, 2 = split bf16 (fp32 accumulate in TMEM either way)
+  int training = 0;     // 1: keep the activations backward needs and build the backward plan (bf16 or split bf16)
 };
 
 struct ParamInfo {

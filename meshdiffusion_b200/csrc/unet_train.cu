@@ -4,6 +4,10 @@
 // bandwidth kernels (backward.cu). Every forward builder records an emitter on a tape; build() runs the tape in
 // reverse, so tensor lifetimes of the whole forward+backward step are packed into one arena by the same first-fit
 // planner as the inference engine.
+//
+// Operand modes: bf16, or split bf16 (kBF16X3: every activation, gradient and scratch operand is a (hi, lo) pair of
+// bf16 tensors in the row layout of gemm_host.h, forward and backward alike, for fp32-class gradients). Pitches handed
+// between emitters stay logical; byte sizes are multiplied by parts(prec_).
 #include "unet.h"
 #include <cmath>
 #include <cstdlib>
@@ -18,7 +22,7 @@ void UNet::free_act(const TensP& t) {
 GradView UNet::new_grad(int C, int R) {
   GradView g;
   g.buf = std::make_shared<GradBuf>();
-  g.buf->off = arena_.alloc((size_t)cfg_.max_batch * R * R * R * C * 2);
+  g.buf->off = arena_.alloc((size_t)cfg_.max_batch * R * R * R * C * esize(prec_) * parts(prec_));
   g.buf->refs = 1;
   g.ptr = dry_ ? nullptr : arena_base_ + g.buf->off;
   g.ld = C; g.C = C;
@@ -28,7 +32,8 @@ GradView UNet::new_grad(int C, int R) {
 GradView UNet::grad_view(const GradView& g, int c0, int C) {
   GradView v = g;
   v.buf->refs++;
-  v.ptr = dry_ ? nullptr : (char*)g.ptr + (size_t)c0 * 2;
+  // (X3: the lo parts of the view sit one logical row (ld) behind its hi parts, so this offsets both halves)
+  v.ptr = dry_ ? nullptr : (char*)g.ptr + (size_t)c0 * esize(prec_);
   v.C = C;
   if (g.colsum) v.colsum = g.colsum + c0;
   return v;
@@ -150,6 +155,7 @@ void UNet::emit_colsum(const std::string& name, const GradView& t, int R, float*
     a.t = t.ptr; a.ld = t.ld; a.C = t.C; a.voxels = (long long)R * R * R;
     a.part = (float*)part.ptr; a.per = per; a.per_ld = per_ld;
     a.from_per = t.colsum; a.from_ld = t.cs_ld;
+    a.x3 = prec_ == kBF16X3 ? 1 : 0;
     add_bwd(name, [=](cudaStream_t s, int B) {
       ColsumArgs c = a;
       c.total0 = g0 >= 0 ? rt_grads_ + g0 : nullptr;
@@ -170,7 +176,7 @@ void UNet::emit_wgrad(const std::string& name, const Act& dy, const Act& x, int 
   if (!dry_) {
     auto op = std::make_unique<WgradOp>();
     op->name = name;
-    op->init(dy, x, ksize, stride, layout, (float*)sc.ptr);
+    op->init(dy, x, ksize, stride, layout, (float*)sc.ptr, prec_ == kBF16X3);
     WgradOp* raw = op.get();
     wgrads_.push_back(std::move(op));
     const bool fixed = dy.B == 1 && cfg_.max_batch != 1;  // batch-reduced operand (mask_layer)
@@ -292,6 +298,7 @@ GradView UNet::emit_gn_backward(const std::string& pname, const std::vector<Tens
     a.add0 = add0 ? add0->ptr : nullptr; a.add0_ld = add0 ? add0->ld : 0;
     a.add1 = add1 ? add1->ptr : nullptr; a.add1_ld = add1 ? add1->ld : 0;
     a.cs_part = (float*)cs_part.ptr; a.cs_per = dx.colsum;
+    a.x3 = prec_ == kBF16X3 ? 1 : 0;
     const long long gw = G(pname + ".weight"), gb = G(pname + ".bias");
     auto with_rt = [this, a, gw, gb, drop_layer]() {
       GnBwdArgs c = a;
@@ -414,6 +421,17 @@ void UNet::tape_attn(TensP x, TensP hn, TensP qkv, TensP S, TensP O, TensP out, 
       return a;
     };
     const float alpha = 1.0f / std::sqrt((float)C);
+    const bool x3 = prec_ == kBF16X3;
+    const size_t pp = parts(prec_);
+    // transposed copy out[b][c][v] = in[b][v][c0 + c] of an operand matrix; X3: rows [ld hi | ld lo] -> [V hi | V lo]
+    auto transpose = [x3, V](const void* in, long long ld, int c0, void* out, int B, int C_, cudaStream_t s) {
+      if (!x3) { launch_transpose_vc(in, ld, c0, out, B, V, C_, 0, s); return; }
+      launch_transpose_vc(in, 2 * ld, c0, out, B, V, C_, 0, s, 2LL * V);
+      launch_transpose_vc(in, 2 * ld, (int)ld + c0, (__nv_bfloat16*)out + V, B, V, C_, 0, s, 2LL * V);
+    };
+    // P and dS: probabilities / logit gradients in the activation dtype at the start of rows of V fp32 slots -- a logical
+    // pitch of 2V bf16, or V for X3 (whose [V hi | V lo] rows fill the slots)
+    const long long sld = x3 ? V : 2LL * V;
     GradView dqkv = new_grad(3 * C, R);
     // dP[q][k] = dOo[q][:] . v[k][:]   (fp32, softmax backward then runs in place)
     Tmp dS = tmp_alloc((size_t)mb * V * V * 4);
@@ -426,13 +444,13 @@ void UNet::tape_attn(TensP x, TensP hn, TensP qkv, TensP S, TensP O, TensP out, 
       add_bwd(g->name, [g](cudaStream_t s, int B) { g->launch(s, B); });
     }
     // dv[k][c] = sum_q P[q][k] dOo[q][c]
-    Tmp PT = tmp_alloc((size_t)mb * V * V * 2);
-    Tmp dOT = tmp_alloc((size_t)mb * C * V * 2);
+    Tmp PT = tmp_alloc((size_t)mb * V * V * 2 * pp);
+    Tmp dOT = tmp_alloc((size_t)mb * C * V * 2 * pp);
     if (!dry_) {
       const void* sp = S->ptr; void* pt = PT.ptr; const void* dop = dOo.ptr; void* dot = dOT.ptr;
       add_bwd(nm + ".PT", [=](cudaStream_t s, int B) {
-        launch_transpose_vc(sp, 2 * V, 0, pt, B, V, V, 0, s);
-        launch_transpose_vc(dop, C, 0, dot, B, V, C, 0, s);
+        transpose(sp, sld, 0, pt, B, V, s);
+        transpose(dop, C, 0, dot, B, C, s);
       });
       GemmOp* g = new_bwd_gemm(nm + ".dv");
       g->set_output_strided(prec_, V, 1, 1, mb, C, (char*)dqkv.ptr + (size_t)2 * C * 2, 3 * C, 0, 0, (long long)V * 3 * C, false);
@@ -440,27 +458,28 @@ void UNet::tape_attn(TensP x, TensP hn, TensP qkv, TensP S, TensP O, TensP out, 
       g->set_b_activation(dOT.ptr, V, C, mb, V, (long long)C * V);
       g->finalize(0, false);
       add_bwd(g->name, [g](cudaStream_t s, int B) { g->launch(s, B); });
-      float* dsp = (float*)dS.ptr; const float* pp = (const float*)S->ptr;
-      add_bwd(nm + ".softmax_bwd", [=](cudaStream_t s, int B) { launch_softmax_bwd_rows(pp, dsp, (long long)B * V, V, s); });
+      float* dsp = (float*)dS.ptr; const float* Pp = (const float*)S->ptr;
+      const int xm = x3 ? 1 : 0;
+      add_bwd(nm + ".softmax_bwd", [=](cudaStream_t s, int B) { launch_softmax_bwd_rows(Pp, dsp, (long long)B * V, V, xm, s); });
     }
     tmp_free(PT);
     tmp_free(dOT);
     unref(dOo);
     free_act(S);
     // dq = alpha dS . k ; dk = alpha dS^T . q
-    Tmp kT = tmp_alloc((size_t)mb * C * V * 2);
-    Tmp qT = tmp_alloc((size_t)mb * C * V * 2);
-    Tmp dST = tmp_alloc((size_t)mb * V * V * 2);
+    Tmp kT = tmp_alloc((size_t)mb * C * V * 2 * pp);
+    Tmp qT = tmp_alloc((size_t)mb * C * V * 2 * pp);
+    Tmp dST = tmp_alloc((size_t)mb * V * V * 2 * pp);
     if (!dry_) {
       const void* qp = qkv->ptr; void* ktp = kT.ptr; void* qtp = qT.ptr; const void* dsp = dS.ptr; void* dstp = dST.ptr;
       add_bwd(nm + ".kT", [=](cudaStream_t s, int B) {
-        launch_transpose_vc(qp, 3 * C, C, ktp, B, V, C, 0, s);
-        launch_transpose_vc(qp, 3 * C, 0, qtp, B, V, C, 0, s);
-        launch_transpose_vc(dsp, 2 * V, 0, dstp, B, V, V, 0, s);
+        transpose(qp, 3 * C, C, ktp, B, C, s);
+        transpose(qp, 3 * C, 0, qtp, B, C, s);
+        transpose(dsp, sld, 0, dstp, B, V, s);
       });
       GemmOp* g = new_bwd_gemm(nm + ".dq");
       g->set_output_strided(prec_, V, 1, 1, mb, C, dqkv.ptr, 3 * C, 0, 0, (long long)V * 3 * C, false);
-      g->add_pointwise({mat(dS.ptr, V, 2 * V)}, nullptr, true);
+      g->add_pointwise({mat(dS.ptr, V, sld)}, nullptr, true);
       g->set_b_activation(kT.ptr, V, C, mb, V, (long long)C * V);
       g->set_alpha(alpha);
       g->finalize(0, false);
@@ -518,7 +537,8 @@ void UNet::tape_downsample(TensP x, TensP out, int midx) {
     GradView z = new_grad(C, Ri);
     if (!dry_) {
       const void* src = dO.ptr; void* dst = z.ptr;
-      add_bwd(nm + ".zero_stuff", [=](cudaStream_t s, int B) { launch_zero_stuff2x(src, dst, B, Ro, C, s); });
+      const int Cp = C * parts(prec_);  // X3: whole (hi, lo) rows
+      add_bwd(nm + ".zero_stuff", [=](cudaStream_t s, int B) { launch_zero_stuff2x(src, dst, B, Ro, Cp, s); });
     }
     GradView prev = x->grad;
     GradView dx = emit_conv_dgrad(nm + ".dgrad", z, Ri, w, C, prev.valid() ? &prev : nullptr);
@@ -546,8 +566,8 @@ void UNet::tape_upsample(TensP x, TensP up, TensP out, int midx) {
     unref(out->grad);
     GradView dx = new_grad(C, x->R);
     if (!dry_) {
-      const void* src = dup.ptr; void* dst = dx.ptr; const int r = x->R;
-      add_bwd(nm + ".downsum", [=](cudaStream_t s, int B) { launch_downsum2x(src, dst, B, r, C, s); });
+      const void* src = dup.ptr; void* dst = dx.ptr; const int r = x->R; const int xm = prec_ == kBF16X3 ? 1 : 0;
+      add_bwd(nm + ".downsum", [=](cudaStream_t s, int B) { launch_downsum2x(src, dst, B, r, C, xm, s); });
     }
     unref(dup);
     if (x->grad.valid()) throw std::runtime_error("mdb: upsample input already has a gradient");
@@ -566,10 +586,11 @@ void UNet::tape_stem(TensP h0, void* Am, int Kpad, int Kpad_m) {
     // h0 = conv(x) + b + pos_layer.bias + mask_layer(mask): the three biases receive the same column sum
     emit_colsum("stem.dbias", dh, R0, nullptr, 0, G("all_modules.2.bias"), cfg_.use_pos_bias ? G("pos_layer.bias") : -1, G("mask_layer.bias"));
     // stem weight: dW[co][ci*T + tap] = sum_v dh[v][co] im2col(x)[v][ci*T + tap]  (im2col recomputed)
-    Tmp A0 = tmp_alloc((size_t)cfg_.max_batch * V0 * Kpad * 2);
+    const int mode = (int)prec_;
+    Tmp A0 = tmp_alloc((size_t)cfg_.max_batch * V0 * Kpad * 2 * parts(prec_));
     if (!dry_) {
       void* a0 = A0.ptr;
-      add_bwd("stem.im2col", [=](cudaStream_t s, int B) { launch_im2col(rt_x_, a0, B, Cin, R0, k, Kpad, 0, s); });
+      add_bwd("stem.im2col", [=](cudaStream_t s, int B) { launch_im2col(rt_x_, a0, B, Cin, R0, k, Kpad, mode, s); });
     }
     {
       Act xa; xa.ptr = A0.ptr; xa.C = Kpad; xa.X = xa.Y = xa.Z = R0; xa.B = cfg_.max_batch;
@@ -578,10 +599,10 @@ void UNet::tape_stem(TensP h0, void* Am, int Kpad, int Kpad_m) {
     }
     tmp_free(A0);
     // mask_layer weight: the mask is shared by the batch -> reduce dh over the batch first
-    Tmp hs = tmp_alloc((size_t)V0 * nf * 2);
+    Tmp hs = tmp_alloc((size_t)V0 * nf * 2 * parts(prec_));
     if (!dry_) {
-      const void* src = dh.ptr; void* dst = hs.ptr;
-      add_bwd("stem.batch_sum", [=](cudaStream_t s, int B) { launch_batch_sum(src, dst, B, V0 * nf, s); });
+      const void* src = dh.ptr; void* dst = hs.ptr; const int xm = prec_ == kBF16X3 ? 1 : 0;
+      add_bwd("stem.batch_sum", [=](cudaStream_t s, int B) { launch_batch_sum(src, dst, B, V0 * nf, nf, xm, s); });
     }
     {
       Act da; da.ptr = hs.ptr; da.C = nf; da.X = da.Y = da.Z = R0; da.B = 1;
@@ -607,10 +628,10 @@ void UNet::tape_head(TensP h, TensP a, const std::string& gn_name, const std::st
     // im2col of dL/dout ([voxel][co*T + tap'], reading dout at v + off(tap')) serves both gradients:
     //   dW[co][c][T-1-tap'] = sum_v a[v][c] Ad[v][co*T + tap'],   da[v][c] = sum_k Ad[v][k] W[co][c][T-1-tap']
     const int Kp = ((Cin * T + 63) / 64) * 64;
-    Tmp Ad = tmp_alloc((size_t)cfg_.max_batch * V0 * Kp * 2);
+    Tmp Ad = tmp_alloc((size_t)cfg_.max_batch * V0 * Kp * 2 * parts(prec_));
     if (!dry_) {
-      void* ad = Ad.ptr;
-      add_bwd("head.im2col", [=](cudaStream_t s, int B) { launch_im2col(rt_dout_, ad, B, Cin, R0, k, Kp, 0, s); });
+      void* ad = Ad.ptr; const int mode = (int)prec_;
+      add_bwd("head.im2col", [=](cudaStream_t s, int B) { launch_im2col(rt_dout_, ad, B, Cin, R0, k, Kp, mode, s); });
     }
     Act ada; ada.ptr = Ad.ptr; ada.C = Kp; ada.X = ada.Y = ada.Z = R0; ada.B = cfg_.max_batch;
     {

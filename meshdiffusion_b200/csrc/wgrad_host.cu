@@ -34,8 +34,8 @@ WgradPlan plan_wgrad(int X, int Y, int Z, int B, int M, int N, int ksize, int st
   return pl;
 }
 
-void WgradOp::init(const Act& dy, const Act& x, int ksize, int stride, const WgradOut& out, float* scratch) {
-  dy_ = dy; x_ = x; ksize_ = ksize; stride_ = stride; out_ = out;
+void WgradOp::init(const Act& dy, const Act& x, int ksize, int stride, const WgradOut& out, float* scratch, bool x3) {
+  dy_ = dy; x_ = x; ksize_ = ksize; stride_ = stride; out_ = out; x3_ = x3;
   M_ = dy.C; N_ = x.C;
   plan_ = plan_wgrad(dy.X, dy.Y, dy.Z, dy.B, M_, N_, ksize, stride);
   if (ksize == 3 && stride == 1 && (x.X != dy.X || x.Y != dy.Y || x.Z != dy.Z)) throw std::runtime_error("mdb: wgrad extent mismatch");
@@ -47,6 +47,8 @@ void WgradOp::init(const Act& dy, const Act& x, int ksize, int stride, const Wgr
   p.taps = plan_.taps;
   p.Mp = plan_.m_tiles * 128; p.Np = plan_.n_tiles * 128;
   p.partial = scratch;
+  p.y_lo = x3 ? (int)dy.row() : 0;
+  p.x_lo = x3 ? (int)x.row() : 0;
   { const char* f = getenv("MDB_WG_DBG"); p.dbg = f ? atoi(f) : 0; }
   p.n_groups = plan_.n_groups;
   const int xrows = plan_.halo ? p.bx * (p.by + 2) : 128;
@@ -71,7 +73,7 @@ void WgradOp::init(const Act& dy, const Act& x, int ksize, int stride, const Wgr
           else p.groups[g++] = WgradGroup{(int8_t)((kx & 1) | ((ky & 1) << 1) | ((kz & 1) << 2)), (int8_t)(kx >> 1), (int8_t)(ky >> 1), (int8_t)(kz >> 1), 1, {tap, 0, 0}};
         }
   }
-  flops = 2.0 * dy.voxels() * dy.B * (double)M_ * N_ * plan_.taps;
+  flops = 2.0 * dy.voxels() * dy.B * (double)M_ * N_ * plan_.taps;  // algorithmic (X3 issues 3x the MMAs)
 }
 
 const WgradParams& WgradOp::params_for(int B) {
@@ -79,14 +81,17 @@ const WgradParams& WgradOp::params_for(int B) {
   if (it != cache_.end()) return it->second;
   WgradParams p = base_;
   const long long es = 2;
+  // X3: a row is [ld hi | ld lo]; the map's channel extent reaches from the view's first hi channel to its last lo one
+  const long long pp = x3_ ? 2 : 1;
+  auto cdim = [&](const Act& a) { return (uint64_t)(x3_ ? a.row() + a.C : a.C); };
   uint64_t dims[5], strides[4];
   uint32_t box[5];
   if (plan_.flat) {
     const long long rows = (long long)B * dy_.voxels();
     p.tx = (int)((rows + 127) / 128); p.ty = p.tz = p.tb = 1;
     auto enc = [&](CUtensorMap* m, const Act& a) {
-      dims[0] = a.C; dims[1] = rows; dims[2] = dims[3] = dims[4] = 1;
-      strides[0] = a.row() * es; strides[1] = strides[0] * rows; strides[2] = strides[1]; strides[3] = strides[1];
+      dims[0] = cdim(a); dims[1] = rows; dims[2] = dims[3] = dims[4] = 1;
+      strides[0] = pp * a.row() * es; strides[1] = strides[0] * rows; strides[2] = strides[1]; strides[3] = strides[1];
       box[0] = 64; box[1] = 128; box[2] = box[3] = box[4] = 1;
       encode_map(m, kBF16, 5, a.ptr, dims, strides, box);
     };
@@ -97,8 +102,8 @@ const WgradParams& WgradOp::params_for(int B) {
     p.tb = (B + p.bb - 1) / p.bb;
     auto enc = [&](CUtensorMap* m, const Act& a, int halo, int sub, int px, int py, int pz) {
       char* base = static_cast<char*>(a.ptr);
-      const long long sx = a.row() * es, sy = sx * a.X, sz = sy * a.Y, sb = sz * a.Z;
-      dims[0] = a.C; dims[4] = B;
+      const long long sx = pp * a.row() * es, sy = sx * a.X, sz = sy * a.Y, sb = sz * a.Z;
+      dims[0] = cdim(a); dims[4] = B;
       if (sub == 1) {
         dims[1] = a.X; dims[2] = a.Y; dims[3] = a.Z;
         strides[0] = sx; strides[1] = sy; strides[2] = sz; strides[3] = sb;
@@ -162,11 +167,13 @@ void WgradOp::launch(cudaStream_t s, int B, bool accumulate, float* out_ptr) {
   MDB_CUDA_CHECK(cudaGetDevice(&dev));
   bool& configured = configured_dev[dev < 64 ? dev : 63];
   if (!configured || dev >= 63) {
-    MDB_CUDA_CHECK(cudaFuncSetAttribute(wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmemBytes));
+    MDB_CUDA_CHECK(cudaFuncSetAttribute(wgrad_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmemBytes));
+    MDB_CUDA_CHECK(cudaFuncSetAttribute(wgrad_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmemBytes));
     configured = true;
   }
   const int grid = p.m_tiles * p.n_tiles * p.n_groups * p.splits;
-  wgrad_tc_kernel<<<grid, kWgThreads, kWgSmemBytes, s>>>(p);
+  if (x3_) wgrad_tc_kernel<true><<<grid, kWgThreads, kWgSmemBytes, s>>>(p);
+  else wgrad_tc_kernel<false><<<grid, kWgThreads, kWgSmemBytes, s>>>(p);
   MDB_CUDA_CHECK(cudaGetLastError());
   WgradReduceArgs r{};
   r.partial = p.partial; r.splits = p.splits; r.taps = p.taps; r.Mp = p.Mp; r.Np = p.Np; r.M = out_.m_valid ? out_.m_valid : M_; r.N = out_.n_valid ? out_.n_valid : N_;

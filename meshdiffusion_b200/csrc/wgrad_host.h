@@ -34,7 +34,8 @@ class WgradOp {
   double flops = 0;
   // dy: [B][Z][Y][X][M] (C = M), x: the forward op's input activation (C = N; for stride 2 at twice the extents).
   // ksize 1 (pointwise; any stride-1 geometry, positions are flattened) or 3 (stride 1 pad 1, or stride 2 pad-high).
-  void init(const Act& dy, const Act& x, int ksize, int stride, const WgradOut& out, float* scratch);
+  // x3: both operands are split-bf16 tensors ((hi, lo) rows of logical pitch ld, gemm_host.h::kBF16X3)
+  void init(const Act& dy, const Act& x, int ksize, int stride, const WgradOut& out, float* scratch, bool x3 = false);
   // accumulate: out += G instead of out = G (micro-batch gradient accumulation)
   void launch(cudaStream_t s, int B, bool accumulate, float* out_ptr = nullptr);
   const WgradPlan& plan() const { return plan_; }
@@ -44,6 +45,7 @@ class WgradOp {
   WgradParams base_{};
   Act dy_, x_;
   int ksize_ = 1, stride_ = 1, M_ = 0, N_ = 0;
+  bool x3_ = false;
   WgradOut out_;
   std::map<int, WgradParams> cache_;  // tensor maps encoded for a given runtime batch
   const WgradParams& params_for(int B);

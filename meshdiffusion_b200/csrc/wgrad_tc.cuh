@@ -50,6 +50,9 @@ struct WgradParams {
   int Mp, Np;           // padded extents (multiples of 128)
   float* partial;       // [splits][taps][Mp][Np]
   int dbg;              // bring-up switch (MDB_WG_DBG): bit 0 swaps the roles of LBO and SBO in the operand descriptors
+  // X3 (split-bf16 operands): the tensor maps span the physical (hi, lo) rows, so the lo parts are the same maps at
+  // channel coordinate +y_lo / +x_lo (the logical row pitches)
+  int y_lo, x_lo;
 };
 
 #ifdef MDB_WGRAD_KERNEL_IMPL  // the kernel itself is compiled in wgrad_host.cu only
@@ -67,7 +70,11 @@ __device__ __forceinline__ void umma_full(uint32_t d_tmem, uint32_t a_lo, uint32
       :: "r"(d_tmem), "r"(a_lo), "r"(b_lo), "r"(idesc), "r"(accumulate), "r"(a_hi), "r"(b_hi) : "memory");
 }
 
+// X3: G = dY_hi.X_hi + dY_hi.X_lo + dY_lo.X_hi into the same accumulators -- every voxel tile is staged three times,
+// (hi, lo), (lo, hi), (hi, hi) (small terms first), with the bytes per MMA of the bf16 kernel
+template <bool X3>
 __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_constant__ WgradParams p) {
+  constexpr int kPasses = X3 ? 3 : 1;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kWgStages * kWgStageBytes);
@@ -111,8 +118,10 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
     // ------------------------------------------------------------------ TMA producer
     uint32_t st = 0, ph = 0;
     const uint32_t bytes = 2 * kWgYChunkBytes + 2 * p.x_chunk_bytes;
-    for (int t = t_lo; t < t_hi; ++t) {
-      int r = t;
+    for (int it = t_lo * kPasses; it < t_hi * kPasses; ++it) {
+      int r = X3 ? it / kPasses : it;
+      const int pass = X3 ? it % kPasses : 0;
+      const int ym = m0 + (pass == 1 ? p.y_lo : 0), xn = n0 + (pass == 0 && X3 ? p.x_lo : 0);
       const int x0 = (r % p.tx) * p.bx; r /= p.tx;
       const int y0 = (r % p.ty) * p.by; r /= p.ty;
       const int z0 = (r % p.tz) * p.bz; r /= p.tz;
@@ -122,11 +131,11 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
         const uint32_t bar = full + 8 * st;
         const uint32_t sbase = stage0 + st * kWgStageBytes;
         mbar_expect_tx(bar, bytes);
-        tma_load_5d(&p.ymap, bar, sbase, m0, x0, y0, z0, b0);
-        tma_load_5d(&p.ymap, bar, sbase + kWgYChunkBytes, m0 + 64, x0, y0, z0, b0);
+        tma_load_5d(&p.ymap, bar, sbase, ym, x0, y0, z0, b0);
+        tma_load_5d(&p.ymap, bar, sbase + kWgYChunkBytes, ym + 64, x0, y0, z0, b0);
         const uint32_t xb = sbase + 2 * kWgYChunkBytes;
-        tma_load_5d(&p.xmap[grp.xmap], bar, xb, n0, x0 + grp.dx, y0 + grp.dy, z0 + grp.dz, b0);
-        tma_load_5d(&p.xmap[grp.xmap], bar, xb + p.x_chunk_bytes, n0 + 64, x0 + grp.dx, y0 + grp.dy, z0 + grp.dz, b0);
+        tma_load_5d(&p.xmap[grp.xmap], bar, xb, xn, x0 + grp.dx, y0 + grp.dy, z0 + grp.dz, b0);
+        tma_load_5d(&p.xmap[grp.xmap], bar, xb + p.x_chunk_bytes, xn + 64, x0 + grp.dx, y0 + grp.dy, z0 + grp.dz, b0);
       }
       __syncwarp();
       if (++st == kWgStages) { st = 0; ph ^= 1; }
@@ -135,14 +144,14 @@ __global__ void __launch_bounds__(kWgThreads, 1) wgrad_tc_kernel(const __grid_co
     // ------------------------------------------------------------------ MMA issuer
     constexpr uint32_t idesc = make_idesc(false, 128, 128) | (1u << 15) | (1u << 16);  // A and B MN-major
     uint32_t st = 0, ph = 0;
-    for (int t = t_lo; t < t_hi; ++t) {
+    for (int it = t_lo * kPasses; it < t_hi * kPasses; ++it) {
       mbar_wait(full + 8 * st, ph);
       tc_fence_after();
       if (elect_one()) {
         const uint32_t sbase = stage0 + st * kWgStageBytes;
         const uint32_t a0 = desc_lo_lbo(sbase, kWgYChunkBytes);
         const uint32_t b0 = desc_lo_lbo(sbase + 2 * kWgYChunkBytes, p.x_chunk_bytes);
-        const uint32_t first = t != t_lo ? 1u : 0u;
+        const uint32_t first = it != t_lo * kPasses ? 1u : 0u;
         if (p.dbg & 1) {
           const uint32_t hi_common = (1u << 14) | (2u << 29);
           const uint32_t a_sw = desc_lo_lbo(sbase, 1024), b_sw = desc_lo_lbo(sbase + 2 * kWgYChunkBytes, 1024);

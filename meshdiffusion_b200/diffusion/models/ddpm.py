@@ -19,6 +19,7 @@ from . import utils
 
 
 PRECISIONS = {"bf16": 0, "tf32": 1, "bf16x3": 2}  # include/meshdiff_b200.h: mdb_unet_config.precision
+TRAIN_PRECISIONS = ("bf16", "bf16x3")  # the engine builds no tf32 training plan
 
 
 def arch_from_config(config):
@@ -123,10 +124,16 @@ class ScoreNet(nn.Module):
         super().__init__()
         self.arch = arch_from_config(config)
         # inference operand mode; the default is the parity-grade one (results within 1e-3 of the reference's fp32 arithmetic).
-        # 'tf32' (1.6e-3, 1.55x faster) and 'bf16' (1.3e-2, 2.7x faster) are opt-in. Training always runs the bf16 plan.
+        # 'tf32' (1.6e-3, 1.55x faster) and 'bf16' (1.3e-2, 2.7x faster) are opt-in.
         self.precision = str(config.model.get("compute_dtype", "bf16x3")) if hasattr(config.model, "get") else "bf16x3"
         if self.precision not in PRECISIONS:
             raise ValueError("config.model.compute_dtype must be 'bf16', 'tf32' or 'bf16x3'")
+        # training operand mode: 'bf16' (the default) or 'bf16x3' (split bf16 forward, data and weight gradients:
+        # fp32-class gradients at about a third of the bf16 tensor rate)
+        training = getattr(config, "training", None)
+        self.train_precision = str(training.get("compute_dtype", "bf16")) if hasattr(training, "get") else "bf16"
+        if self.train_precision not in TRAIN_PRECISIONS:
+            raise ValueError("config.training.compute_dtype must be 'bf16' or 'bf16x3'")
         self.max_batch = int(config.model.get("engine_max_batch", 0) or 0) if hasattr(config.model, "get") else 0
         self.scale_by_sigma = bool(config.model.scale_by_sigma)
         self.dropout = float(config.model.get("dropout", 0.0)) if hasattr(config.model, "get") else 0.0
@@ -215,7 +222,7 @@ class ScoreNet(nn.Module):
             _native.lib().mdb_unet_destroy(self._train_handle)
             self._train_handle = None
 
-    # ---- training engine (bf16 operands, fp32 master parameters and gradients) ------------------------------------
+    # ---- training engine (bf16 or split-bf16 operands, fp32 master parameters and gradients) ----------------------
     def _ensure_train_engine(self, batch, device):
         L = _native.lib()
         if self._train_handle is not None and batch <= self._train_batch:
@@ -225,7 +232,7 @@ class ScoreNet(nn.Module):
         if self._train_handle is not None:
             L.mdb_unet_destroy(self._train_handle)
             self._train_handle = None
-        cfg = _config_c(self.arch, batch, "bf16", training=True)
+        cfg = _config_c(self.arch, batch, self.train_precision, training=True)
         h = ctypes.c_void_p()
         with torch.cuda.device(device):
             _native.check(L.mdb_unet_create(ctypes.byref(cfg), ctypes.byref(h)))

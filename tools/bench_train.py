@@ -1,7 +1,7 @@
 """Training-step throughput of the PRODUCT training path (BASELINE.json configs[2]: res64 train, synthetic 4x64^3 grids,
 bf16 operands, fp32 master weights + Adam + EMA, data-parallel gradient mean).
 
-    python tools/bench_train.py [--batch 16] [--iters 4] [--steps 3] [--warmup 1]
+    python tools/bench_train.py [--batch 16] [--iters 4] [--steps 3] [--warmup 1] [--precision bf16|bf16x3]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P tools/bench_train.py ...
 
 The step that is timed is the one `main_diffusion.py --mode=train` runs: trainer.build_state / trainer.make_train_step ->
@@ -9,7 +9,8 @@ losses.get_step_fn (native perturb + loss node, engine forward / backward throug
 overlapped with the backward pass, FusedAdam with clip coefficient + EMA in one pass). One optimiser step = `iters`
 micro-batches of `batch` grids per GPU. Prints ONE JSON line: samples/s over all ranks, the device-time split (CUDA events
 around the product methods; `allreduce` is the EXPOSED wait of the optimiser on the side-stream reductions) and the achieved
-tensor-core rate (forward + backward GEMM FLOPs / their device time) against the measured sustained bf16 peak.
+tensor-core rate (forward + backward GEMM FLOPs / their device time) against the measured sustained bf16 peak (divided by
+the 3 MMAs per product in the split-bf16 mode, `--precision bf16x3`, as bench.py does), and the engine's arena size.
 """
 import argparse
 import ctypes
@@ -24,11 +25,15 @@ os.environ.setdefault("NCCL_DEBUG", "WARN")
 import torch  # noqa: E402
 
 
-def run(batch=16, iters=4, steps=3, warmup=1, config="res64", dropout=0.1, no_overlap=False, profile=None):
+MMA_PER_PRODUCT = {"bf16": 1.0, "bf16x3": 3.0}
+
+
+def run(batch=16, iters=4, steps=3, warmup=1, config="res64", dropout=0.1, no_overlap=False, profile=None, precision="bf16"):
     """Runs the measurement on every rank (joins the NCCL group if the caller has not) and returns the JSON line as a dict
-    on rank 0 (None elsewhere). bench.py calls this in-process for its `train` leg."""
+    on rank 0 (None elsewhere). bench.py calls this in-process for its `train` leg. `precision`: the training operand mode
+    (config.training.compute_dtype)."""
     args = argparse.Namespace(batch=batch, iters=iters, steps=steps, warmup=warmup, config=config, dropout=dropout,
-                              no_overlap=no_overlap, profile=profile)
+                              no_overlap=no_overlap, profile=profile, precision=precision)
     import torch.distributed as dist
     from configs import res64, res128
     from meshdiffusion_b200 import _native
@@ -50,6 +55,7 @@ def run(batch=16, iters=4, steps=3, warmup=1, config="res64", dropout=0.1, no_ov
         cfg.data.image_size, cfg.model.nf, cfg.model.ch_mult = 16, 32, (1, 2)
         cfg.model.num_res_blocks, cfg.model.attn_resolutions = 1, (8,)
     cfg.model.compute_dtype = "bf16"
+    cfg.training.compute_dtype = args.precision
     cfg.model.dropout = args.dropout
     cfg.training.iter_size = args.iters
     cfg.device = dev
@@ -141,8 +147,8 @@ def run(batch=16, iters=4, steps=3, warmup=1, config="res64", dropout=0.1, no_ov
     split["allreduce_exposed"] = sum(a.elapsed_time(b) for k, a, b in marks if k == "allreduce_exposed")
     split["other (loss, clip, Adam+EMA, host gaps)"] = ms - sum(split.values())
     L = _native.lib()
-    fl, bf, nb, numel = ctypes.c_double(), ctypes.c_double(), ctypes.c_int(), ctypes.c_longlong()
-    _native.check(L.mdb_unet_info(net._train_handle, ctypes.byref(fl), None, None, None))
+    fl, bf, nb, numel, arena = ctypes.c_double(), ctypes.c_double(), ctypes.c_int(), ctypes.c_longlong(), ctypes.c_longlong()
+    _native.check(L.mdb_unet_info(net._train_handle, ctypes.byref(fl), ctypes.byref(arena), None, None))
     _native.check(L.mdb_unet_train_info(net._train_handle, ctypes.byref(bf), ctypes.byref(nb), ctypes.byref(numel)))
     samples = args.steps * args.iters * B * world
     peak = 1418.0
@@ -150,6 +156,7 @@ def run(batch=16, iters=4, steps=3, warmup=1, config="res64", dropout=0.1, no_ov
         peak = float(json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))["bf16_tflops_sustained"])
     except Exception:
         pass
+    peak /= MMA_PER_PRODUCT[args.precision]  # algorithmic FLOPs: the split mode issues 3 MMAs per product
     tc_ms = split["fwd"] + split["bwd"]
     achieved = (fl.value + bf.value) * args.steps * args.iters * B / (tc_ms * 1e-3) / 1e12 if tc_ms > 0 else None
     if args.profile and rank == 0:
@@ -166,9 +173,9 @@ def run(batch=16, iters=4, steps=3, warmup=1, config="res64", dropout=0.1, no_ov
     result = None
     if rank == 0:
         result = ({
-            "metric": "training samples/s (res64 4x64^3 grids, bf16 operands, fp32 master/Adam/EMA)", "value": samples / (ms * 1e-3),
+            "metric": f"training samples/s (res64 4x64^3 grids, {args.precision} operands, fp32 master/Adam/EMA)", "value": samples / (ms * 1e-3),
             "unit": "samples/s", "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms / args.steps,
-            "higher_is_better": True, "scaling": "weak", "dtype": "bf16", "data": "synthetic",
+            "higher_is_better": True, "scaling": "weak", "dtype": args.precision, "data": "synthetic",
             "path": "product: trainer.make_train_step -> losses.get_step_fn -> FusedAdam(+EMA); all-reduce " +
                     ("blocking" if args.no_overlap else f"bucketed ({len(net._grad_buckets()) if world > 1 else 0} buckets) and overlapped with backward"),
             "config": {"workload": f"{args.config}.py train, micro-batch {B} x {args.iters} per GPU, dropout {args.dropout}, clip 1.0, Adam + EMA",
@@ -176,8 +183,8 @@ def run(batch=16, iters=4, steps=3, warmup=1, config="res64", dropout=0.1, no_ov
             "split_ms_per_step": {k: v / args.steps for k, v in split.items()},
             "flops_per_sample": {"forward": fl.value, "backward": bf.value},
             "roofline": {"bound": "tensor", "achieved": achieved, "peak": peak, "unit": "TFLOP/s", "frac": achieved / peak if achieved else None,
-                         "note": "forward + backward GEMM FLOPs / (fwd + bwd device time)"},
-            "bwd_launches": nb.value, "params": numel.value, "losses": losses,
+                         "note": "forward + backward GEMM FLOPs / (fwd + bwd device time); peak = sustained bf16 / MMAs per product"},
+            "bwd_launches": nb.value, "params": numel.value, "arena_bytes": arena.value, "losses": losses,
         })
     net.release_engine()
     if own_group:
@@ -195,8 +202,9 @@ def main():
     ap.add_argument("--dropout", type=float, default=0.1)
     ap.add_argument("--no-overlap", action="store_true", help="one blocking all-reduce after the backward pass instead of buckets")
     ap.add_argument("--profile", default=None, help="write per-launch device times of one forward+backward as JSON")
+    ap.add_argument("--precision", default="bf16", choices=["bf16", "bf16x3"], help="training operand mode (config.training.compute_dtype)")
     a = ap.parse_args()
-    out = run(a.batch, a.iters, a.steps, a.warmup, a.config, a.dropout, a.no_overlap, a.profile)
+    out = run(a.batch, a.iters, a.steps, a.warmup, a.config, a.dropout, a.no_overlap, a.profile, a.precision)
     if out is not None:
         print(json.dumps(out))
 
