@@ -193,18 +193,60 @@ int mdb_conv3d(const void* x, int batch, int cin, int z, int y_, int x_, const f
 int mdb_groupnorm_act(const void* x, const long long* stats, const float* gamma, const float* beta, void* y, int batch,
                       long long voxels, int channels, int silu, int precision, void* stream);
 
-/* Backward of mdb_conv3d for bf16 operands (k = 3 stride 1 | 2, or k = 1): what autograd's conv3d backward returns.
- * dy: [B][Zo][Yo][Xo][Cout], x: [B][Z][Y][X][Cin] (both bf16 NDHWC), w: fp32 OIDHW. dw (nullable): fp32 OIDHW;
- * dx (nullable, stride 1 only): bf16 [B][Z][Y][X][Cin]. Synchronises. */
+/* Backward of mdb_conv3d (k = 3 stride 1 | 2, or k = 1) in the training operand modes, precision 0 (bf16) or 2 (bf16x3):
+ * what autograd's conv3d backward returns. dy: [B][Zo][Yo][Xo][Cout], x: [B][Z][Y][X][Cin] (NDHWC, operand dtype), w: fp32
+ * OIDHW. dy_ld / x_ld: logical row pitches in channels (0 = dense); a channel view is a pointer offset plus a pitch, and in
+ * bf16x3 its lo half sits one logical row (ld) behind its hi half. dw (nullable): fp32 OIDHW, += when accumulate != 0.
+ * dx (nullable; dense [B][Z][Y][X][Cin], operand dtype): stride 2 is the transposed convolution the training plan runs
+ * (dy zero-stuffed to the input extents, then the stride-1 data gradient; needs dense dy and cubic extents).
+ * batch_plan >= batch (0 = batch): the operations are planned for batch_plan and launched for batch. splits > 1: the data
+ * gradient runs split-K with that factor (fp32 partials + the split reduction); `residual` (nullable, dense like dx) is
+ * added to dx. Synchronises. */
 int mdb_conv3d_backward(const void* dy, const void* x, const float* w, int batch, int cin, int cout, int z, int y_,
-                        int x_, int ksize, int stride, float* dw, void* dx, void* stream);
-/* Backward of mdb_groupnorm_act (bf16): da = dL/dy [B][V][C] -> dx [B][V][C], dgamma / dbeta fp32 [C]. `add`
- * (nullable, [B][V][C]) is summed into dx. Dropout (p, seed) as in mdb_unet_set_dropout. `da` is used as scratch
+                        int x_, int ksize, int stride, float* dw, void* dx, int precision, long long dy_ld, long long x_ld,
+                        int accumulate, int batch_plan, int splits, const void* residual, void* stream);
+/* Backward of mdb_groupnorm_act over the channel concatenation of x0 (c0 channels) and x1 (c1, nullable), precision 0 or 2:
+ * da = dL/dy [B][V][C] (C = c0 + c1) -> dx [B][V][C], dgamma / dbeta fp32 [C] (+= when accumulate != 0). add0 / add1
+ * (nullable, [B][V][C]) are summed into dx. Dropout (p, seed) as in mdb_unet_set_dropout. cs_per (nullable): fp32 [B][C]
+ * per-sample column sums of dx. stats0 / stats1: [B][c0|c1][4] split fixed point, as above. `da` is used as scratch
  * (overwritten with the pre-activation gradient). Synchronises. */
-int mdb_groupnorm_act_backward(const void* x, const long long* stats, const float* gamma, const float* beta,
-                               void* da, const void* add, void* dx, float* dgamma, float* dbeta, int batch,
-                               long long voxels, int channels, int silu, float dropout_p, unsigned long long seed,
-                               void* stream);
+int mdb_groupnorm_act_backward(const void* x0, int c0, const void* x1, int c1, const long long* stats0,
+                               const long long* stats1, const float* gamma, const float* beta, void* da, const void* add0,
+                               const void* add1, void* dx, float* dgamma, float* dbeta, float* cs_per, int batch,
+                               long long voxels, int silu, float dropout_p, unsigned long long seed, int precision,
+                               int accumulate, void* stream);
+/* The fused data-gradient + GroupNorm backward of the training plan: da = the data gradient of a k = 3 (stride 1) or
+ * k = 1 convolution with weight w (fp32 OIDHW [cout][C][k^3]) applied to dy ([B][R^3][cout]), consumed in the GEMM
+ * epilogue as dL/d(output) of GroupNorm(+SiLU)(+dropout) whose input is the concatenation of x0 (c0) and x1 (c1,
+ * nullable); then the per-tile partials are reduced and dx = the GroupNorm input gradient (+ add0 + add1) is applied.
+ * Same outputs as mdb_conv3d_backward's dx followed by mdb_groupnorm_act_backward. Fails if the GEMM's tile plan is not
+ * the one the partial buffers were sized for. Synchronises. */
+int mdb_conv3d_dgrad_gn_backward(const void* dy, const float* w, int batch, int cout, int r, int ksize, const void* x0,
+                                 int c0, const void* x1, int c1, const long long* stats0, const long long* stats1,
+                                 const float* gamma, const float* beta, const void* add0, const void* add1, void* dx,
+                                 float* dgamma, float* dbeta, int silu, float dropout_p, unsigned long long seed,
+                                 int precision, void* stream);
+/* Bandwidth kernels of the training backward, one launch each (precision 0 = bf16, 2 = bf16x3 (hi, lo) rows). Synchronise.
+ * colsum: per [B][per_ld] (nullable) = sum_v t[b][v][c]; total [C] (nullable; += when accumulate) = sum_b per. t has logical
+ * pitch ld >= C. from_per (nullable, [B][from_ld] fp32): per-sample sums already computed; only the batch sum runs. */
+int mdb_colsum(const void* t, long long ld, int channels, int batch, long long voxels, float* per, long long per_ld,
+               float* total, int accumulate, const float* from_per, long long from_ld, int precision, void* stream);
+/* Upsample backward: dx [B][R^3][C] = sum over each 2x2x2 block of dup [B][(2R)^3][C]. */
+int mdb_downsum2x(const void* dup, void* dx, int batch, int r, int channels, int precision, void* stream);
+/* out [V][C] = sum_b t[b][v][c]. */
+int mdb_batch_sum(const void* t, void* out, int batch, long long voxels, int channels, int precision, void* stream);
+/* Downsample backward helper: z [B][(2R)^3][C] = dy [B][R^3][C] at the odd sites of every axis, zero elsewhere. */
+int mdb_zero_stuff2x(const void* dy, void* z, int batch, int r, int channels, int precision, void* stream);
+/* Attention softmax backward in place: rows of L fp32 slots; P holds the probabilities as the forward softmax leaves them
+ * (bf16 at the start of each row; bf16x3: L hi then L lo), dP the fp32 upstream gradient; dS = P (dP - sum(P dP)) replaces
+ * dP in the same format as P. */
+int mdb_softmax_bwd_rows(const float* p, float* dp, long long rows, int l, int precision, void* stream);
+/* out[b][c][v] = in[b][v][c0 + c] for c < C, in of logical pitch ld; bf16x3: in rows [ld hi | ld lo] -> out rows
+ * [V hi | V lo] (the attention backward's operand transposes). */
+int mdb_transpose_vc(const void* in, long long ld, int c0, void* out, int batch, int voxels, int channels, int precision,
+                     void* stream);
+/* im2col of fp32 NCDHW x [B][cin][R^3] -> a [B][R^3][kpad] (column cin*k^3 + tap, zero padded), operand dtype. */
+int mdb_im2col(const float* x, void* a, int batch, int cin, int r, int ksize, int kpad, int precision, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
  * Marching tetrahedra. Replaces DMTet.__call__ (nvdiffrec/lib/geometry/dmtet.py:105-163; tables :34-54, map_uv

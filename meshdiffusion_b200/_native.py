@@ -82,8 +82,18 @@ SIGNATURES = {
     "mdb_allreduce_grads": (_i, [_vp, _vp, _ll, _i, _vp]),
     "mdb_conv3d": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _i, _i, _vp, _vp, _vp, _vp, _i, _vp]),
     "mdb_groupnorm_act": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _ll, _i, _i, _i, _vp]),
-    "mdb_conv3d_backward": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp]),
-    "mdb_groupnorm_act_backward": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _ll, _i, _i, _f, _u64, _vp]),
+    "mdb_conv3d_backward": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _i, _ll, _ll, _i, _i, _i, _vp, _vp]),
+    "mdb_groupnorm_act_backward": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _ll, _i, _f, _u64,
+                                        _i, _i, _vp]),
+    "mdb_conv3d_dgrad_gn_backward": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                          _i, _f, _u64, _i, _vp]),
+    "mdb_colsum": (_i, [_vp, _ll, _i, _i, _ll, _vp, _ll, _vp, _i, _vp, _ll, _i, _vp]),
+    "mdb_downsum2x": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
+    "mdb_batch_sum": (_i, [_vp, _vp, _i, _ll, _i, _i, _vp]),
+    "mdb_zero_stuff2x": (_i, [_vp, _vp, _i, _i, _i, _i, _vp]),
+    "mdb_softmax_bwd_rows": (_i, [_vp, _vp, _ll, _i, _i, _vp]),
+    "mdb_transpose_vc": (_i, [_vp, _ll, _i, _vp, _i, _i, _i, _i, _vp]),
+    "mdb_im2col": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "mdb_marching_tets_prepare": (_i, [_vp, _i, _i, _i, ctypes.POINTER(_vp)]),
     "mdb_marching_tets_destroy": (None, [_vp]),
     "mdb_marching_tets_info": (_i, [_vp, ctypes.POINTER(_i), ctypes.POINTER(_i)]),

@@ -3,6 +3,7 @@
 #include "unet.h"
 #include <cstring>
 #include <cmath>
+#include <memory>
 
 using namespace mdb;
 
@@ -304,56 +305,214 @@ int mdb_groupnorm_act(const void* x, const long long* stats, const float* gamma,
   MDB_API_END
 }
 
+// Device scratch of the operator entry points, freed on every exit path.
+struct DevBuf {
+  void* p = nullptr;
+  explicit DevBuf(size_t bytes) { MDB_CUDA_CHECK(cudaMalloc(&p, bytes ? bytes : 16)); }
+  ~DevBuf() { if (p) cudaFree(p); }
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  float* f() const { return static_cast<float*>(p); }
+};
+
+static Precision train_precision(int v) {
+  const Precision p = precision_from_int(v);
+  if (p == kTF32) throw std::runtime_error("mdb: the training kernels take precision 0 (bf16) or 2 (bf16x3)");
+  return p;
+}
+
+static Act act5(const void* ptr, int C, long long ld, int X, int Y, int Z, int B) {
+  Act a;
+  a.ptr = const_cast<void*>(ptr); a.C = C; a.ld = ld; a.X = X; a.Y = Y; a.Z = Z; a.B = B;
+  return a;
+}
+
 int mdb_conv3d_backward(const void* dy, const void* x, const float* w, int B, int cin, int cout, int z, int y_, int x_,
-                        int ksize, int stride, float* dw, void* dx, void* stream) {
+                        int ksize, int stride, float* dw, void* dx, int precision, long long dy_ld, long long x_ld,
+                        int accumulate, int B_plan, int splits, const void* residual, void* stream) {
   MDB_API_BEGIN
   cudaStream_t s = (cudaStream_t)stream;
+  const Precision pr = train_precision(precision);
+  if (B_plan == 0) B_plan = B;
+  if (B < 1 || B_plan < B) throw std::runtime_error("mdb: conv3d backward needs 1 <= batch <= batch_plan");
+  if (stride != 1 && stride != 2) throw std::runtime_error("mdb: conv3d backward supports stride 1 and 2");
   const int xo = x_ / stride, yo = y_ / stride, zo = z / stride;
-  Act ady; ady.ptr = const_cast<void*>(dy); ady.C = cout; ady.X = xo; ady.Y = yo; ady.Z = zo; ady.B = B;
-  Act ax; ax.ptr = const_cast<void*>(x); ax.C = cin; ax.X = x_; ax.Y = y_; ax.Z = z; ax.B = B;
+  const Act ady = act5(dy, cout, dy_ld, xo, yo, zo, B_plan);
+  const Act ax = act5(x, cin, x_ld, x_, y_, z, B_plan);
   if (dw) {
     const int T = ksize * ksize * ksize;
-    const WgradPlan pl = plan_wgrad(xo, yo, zo, B, cout, cin, ksize, stride);
-    float* scratch = nullptr;
-    MDB_CUDA_CHECK(cudaMalloc(&scratch, pl.scratch_bytes));
+    const WgradPlan pl = plan_wgrad(xo, yo, zo, B_plan, cout, cin, ksize, stride);
+    DevBuf scratch(pl.scratch_bytes);
     WgradOut o; o.ptr = dw; o.sm = (long long)cin * T; o.sn = T; o.st = 1;
     WgradOp op;
-    op.init(ady, ax, ksize, stride, o, scratch);
-    op.launch(s, B, false);
+    op.init(ady, ax, ksize, stride, o, scratch.f(), pr == kBF16X3);
+    op.launch(s, B, accumulate != 0);
     MDB_CUDA_CHECK(cudaStreamSynchronize(s));
-    cudaFree(scratch);
   }
   if (dx) {
-    if (stride != 1) throw std::runtime_error("mdb: conv3d data gradient entry point supports stride 1");
+    const long long V = (long long)x_ * y_ * z;
+    Act src = ady;
+    std::unique_ptr<DevBuf> stuffed;
+    if (stride == 2) {
+      // the training plan's transposed stride-2 convolution: dY zero-stuffed to the input extents, then the stride-1
+      // data gradient with the mirrored kernel (UNet::tape_downsample)
+      if (ksize != 3 || (dy_ld && dy_ld != cout) || x_ != y_ || y_ != z)
+        throw std::runtime_error("mdb: stride-2 data gradient needs k = 3, dense dy and cubic extents");
+      stuffed = std::make_unique<DevBuf>((size_t)B_plan * V * cout * 2 * parts(pr));
+      launch_zero_stuff2x(dy, stuffed->p, B, xo, cout * parts(pr), s);
+      src = act5(stuffed->p, cout, 0, x_, y_, z, B_plan);
+    }
     GemmOp g;
-    g.set_output(kBF16, x_, y_, z, B, cin, dx, cin, false);
-    if (ksize == 1) { WSrc ws{w, 1, (long long)cin, 0, cout}; g.add_pointwise_w({ady}, &ws); }
-    else g.add_conv_dgrad(ady, w, cin, ksize);
+    g.set_output(pr, x_, y_, z, B_plan, cin, dx, cin, false);
+    if (ksize == 1) { WSrc ws{w, 1, (long long)cin, 0, cout}; g.add_pointwise_w({src}, &ws); }
+    else g.add_conv_dgrad(src, w, cin, ksize);
+    if (residual) g.set_residual(residual, cin, V * cin, false);
+    std::unique_ptr<DevBuf> partial;
+    if (splits > 1) {
+      partial = std::make_unique<DevBuf>((size_t)splits * B_plan * V * cin * sizeof(float));
+      g.enable_splits(splits, partial->f());
+    }
     g.finalize(s, true);
-    g.launch(s);
+    g.launch(s, B);
     MDB_CUDA_CHECK(cudaStreamSynchronize(s));
   }
   MDB_API_END
 }
 
-int mdb_groupnorm_act_backward(const void* x, const long long* stats, const float* gamma, const float* beta, void* da,
-                               const void* add, void* dx, float* dgamma, float* dbeta, int B, long long V, int C, int silu,
-                               float dropout_p, unsigned long long seed, void* stream) {
-  MDB_API_BEGIN
-  cudaStream_t s = (cudaStream_t)stream;
-  float *part = nullptr, *sums = nullptr;
-  MDB_CUDA_CHECK(cudaMalloc(&part, (size_t)kBwdPartRows(B) * C * 2 * sizeof(float)));
-  MDB_CUDA_CHECK(cudaMalloc(&sums, (size_t)B * C * 2 * sizeof(float)));
+static GnBwdArgs gn_bwd_args(const void* x0, int c0, const void* x1, int c1, const long long* stats0, const long long* stats1,
+                             const float* gamma, const float* beta, const void* add0, const void* add1, void* dx,
+                             float* dgamma, float* dbeta, long long V, int silu, float dropout_p, unsigned long long seed,
+                             Precision pr) {
+  if (dropout_p < 0.f || dropout_p >= 1.f) throw std::runtime_error("mdb: dropout probability out of range");
   GnBwdArgs a{};
-  a.x0 = x; a.C0 = C; a.ld0 = C; a.stats0 = stats; a.gamma = gamma; a.beta = beta; a.da = da;
+  a.x0 = x0; a.C0 = c0; a.ld0 = c0; a.stats0 = stats0;
+  a.x1 = x1; a.C1 = x1 ? c1 : 0; a.ld1 = a.C1; a.stats1 = x1 ? stats1 : nullptr;
+  a.gamma = gamma; a.beta = beta;
   a.voxels = V; a.silu = silu; a.groups = 32; a.eps = 1e-6f;
   a.drop_thresh = (int)lround((double)dropout_p * 65536.0); a.drop_scale = dropout_p > 0.f ? 1.f / (1.f - dropout_p) : 1.f; a.seed = seed;
-  a.part = part; a.sums = sums; a.dgamma = dgamma; a.dbeta = dbeta; a.accumulate = 0;
-  a.dx = dx; a.add0 = add; a.add0_ld = C;
+  a.dgamma = dgamma; a.dbeta = dbeta;
+  const int C = a.C0 + a.C1;
+  a.dx = dx; a.add0 = add0; a.add0_ld = C; a.add1 = add1; a.add1_ld = C;
+  a.x3 = pr == kBF16X3 ? 1 : 0;
+  return a;
+}
+
+int mdb_groupnorm_act_backward(const void* x0, int c0, const void* x1, int c1, const long long* stats0, const long long* stats1,
+                               const float* gamma, const float* beta, void* da, const void* add0, const void* add1, void* dx,
+                               float* dgamma, float* dbeta, float* cs_per, int B, long long V, int silu, float dropout_p,
+                               unsigned long long seed, int precision, int accumulate, void* stream) {
+  MDB_API_BEGIN
+  cudaStream_t s = (cudaStream_t)stream;
+  GnBwdArgs a = gn_bwd_args(x0, c0, x1, c1, stats0, stats1, gamma, beta, add0, add1, dx, dgamma, dbeta, V, silu, dropout_p,
+                            seed, train_precision(precision));
+  const int C = a.C0 + a.C1;
+  DevBuf part((size_t)kBwdPartRows(B) * C * 2 * sizeof(float)), sums((size_t)B * C * 2 * sizeof(float));
+  std::unique_ptr<DevBuf> cs_part;
+  if (cs_per) cs_part = std::make_unique<DevBuf>((size_t)kBwdPartRows(B) * C * sizeof(float));
+  a.da = da; a.part = part.f(); a.sums = sums.f(); a.accumulate = accumulate != 0;
+  a.cs_part = cs_per ? cs_part->f() : nullptr; a.cs_per = cs_per;
   launch_gn_bwd_reduce(a, B, s);
   launch_gn_bwd_apply(a, B, s);
   MDB_CUDA_CHECK(cudaStreamSynchronize(s));
-  cudaFree(part); cudaFree(sums);
+  MDB_API_END
+}
+
+int mdb_conv3d_dgrad_gn_backward(const void* dy, const float* w, int B, int cout, int R, int ksize, const void* x0, int c0,
+                                 const void* x1, int c1, const long long* stats0, const long long* stats1, const float* gamma,
+                                 const float* beta, const void* add0, const void* add1, void* dx, float* dgamma, float* dbeta,
+                                 int silu, float dropout_p, unsigned long long seed, int precision, void* stream) {
+  MDB_API_BEGIN
+  cudaStream_t s = (cudaStream_t)stream;
+  const Precision pr = train_precision(precision);
+  if (ksize != 1 && ksize != 3) throw std::runtime_error("mdb: the fused data gradient supports k = 1 and k = 3");
+  GnBwdArgs a = gn_bwd_args(x0, c0, x1, c1, stats0, stats1, gamma, beta, add0, add1, dx, dgamma, dbeta, (long long)R * R * R,
+                            silu, dropout_p, seed, pr);
+  const int C = a.C0 + a.C1;
+  // partial buffers sized the way UNet::gn_fuse_attach sizes them
+  const Geometry geo = pick_geometry(R, R, R);
+  const int T = ((R + geo.bx - 1) / geo.bx) * ((R + geo.by - 1) / geo.by) * ((R + geo.bz - 1) / geo.bz);
+  const long long rows = 1LL * T * ((B + geo.bb - 1) / geo.bb) * geo.bb;
+  DevBuf consts((size_t)B * C * 4 * sizeof(float)), tile_part((size_t)rows * C * 2 * sizeof(float));
+  DevBuf sums((size_t)B * C * 2 * sizeof(float)), da((size_t)B * a.voxels * C * 2 * parts(pr));
+  a.da = da.p; a.sums = sums.f();
+  GemmOp g;
+  g.set_output(pr, R, R, R, B, C, da.p, C, false);
+  const Act ady = act5(dy, cout, 0, R, R, R, B);
+  if (ksize == 1) { WSrc ws{w, 1, (long long)C, 0, cout}; g.add_pointwise_w({ady}, &ws); }
+  else g.add_conv_dgrad(ady, w, C, 3);
+  g.set_gn_backward(x0, c0, c0, x1, x1 ? c1 : 0, consts.p, silu, tile_part.f());
+  if (g.gnb_tiles_per_batch_tile() != T || g.gnb_bb() != geo.bb || g.gnb_rows() != rows)
+    throw std::runtime_error("mdb: GroupNorm-backward tile plan mismatch");
+  g.rt_drop_thresh = a.drop_thresh; g.rt_drop_scale = a.drop_scale; g.rt_seed = a.seed;
+  g.finalize(s, true);
+  launch_gn_consts(a, consts.f(), B, s);
+  g.launch(s, B);
+  launch_gnb_tile_reduce(a, tile_part.f(), T, geo.bb, B, s);
+  launch_gn_bwd_apply(a, B, s);
+  MDB_CUDA_CHECK(cudaStreamSynchronize(s));
+  MDB_API_END
+}
+
+int mdb_colsum(const void* t, long long ld, int C, int B, long long V, float* per, long long per_ld, float* total,
+               int accumulate, const float* from_per, long long from_ld, int precision, void* stream) {
+  MDB_API_BEGIN
+  cudaStream_t s = (cudaStream_t)stream;
+  DevBuf part((size_t)kBwdPartRows(B) * C * sizeof(float));
+  ColsumArgs a{};
+  a.t = t; a.ld = ld ? ld : C; a.C = C; a.voxels = V; a.part = part.f();
+  a.per = per; a.per_ld = per_ld; a.total0 = total; a.accumulate = accumulate != 0;
+  a.from_per = from_per; a.from_ld = from_ld;
+  a.x3 = train_precision(precision) == kBF16X3 ? 1 : 0;
+  launch_colsum(a, B, s);
+  MDB_CUDA_CHECK(cudaStreamSynchronize(s));
+  MDB_API_END
+}
+
+int mdb_downsum2x(const void* dup, void* dx, int B, int R, int C, int precision, void* stream) {
+  MDB_API_BEGIN
+  cudaStream_t s = (cudaStream_t)stream;
+  launch_downsum2x(dup, dx, B, R, C, train_precision(precision) == kBF16X3 ? 1 : 0, s);
+  MDB_CUDA_CHECK(cudaStreamSynchronize(s));
+  MDB_API_END
+}
+
+int mdb_batch_sum(const void* t, void* out, int B, long long V, int C, int precision, void* stream) {
+  MDB_API_BEGIN
+  cudaStream_t s = (cudaStream_t)stream;
+  launch_batch_sum(t, out, B, V * C, C, train_precision(precision) == kBF16X3 ? 1 : 0, s);
+  MDB_CUDA_CHECK(cudaStreamSynchronize(s));
+  MDB_API_END
+}
+
+int mdb_zero_stuff2x(const void* dy, void* z, int B, int R, int C, int precision, void* stream) {
+  MDB_API_BEGIN
+  cudaStream_t s = (cudaStream_t)stream;
+  launch_zero_stuff2x(dy, z, B, R, C * parts(train_precision(precision)), s);  // whole (hi, lo) rows
+  MDB_CUDA_CHECK(cudaStreamSynchronize(s));
+  MDB_API_END
+}
+
+int mdb_softmax_bwd_rows(const float* P, float* dP, long long rows, int L, int precision, void* stream) {
+  MDB_API_BEGIN
+  cudaStream_t s = (cudaStream_t)stream;
+  launch_softmax_bwd_rows(P, dP, rows, L, train_precision(precision) == kBF16X3 ? 1 : 0, s);
+  MDB_CUDA_CHECK(cudaStreamSynchronize(s));
+  MDB_API_END
+}
+
+int mdb_transpose_vc(const void* in, long long ld, int c0, void* out, int B, int V, int C, int precision, void* stream) {
+  MDB_API_BEGIN
+  cudaStream_t s = (cudaStream_t)stream;
+  launch_transpose_vc_rows(in, ld, c0, out, B, V, C, train_precision(precision) == kBF16X3 ? 1 : 0, s);
+  MDB_CUDA_CHECK(cudaStreamSynchronize(s));
+  MDB_API_END
+}
+
+int mdb_im2col(const float* x, void* a, int B, int cin, int R, int ksize, int kpad, int precision, void* stream) {
+  MDB_API_BEGIN
+  cudaStream_t s = (cudaStream_t)stream;
+  launch_im2col(x, a, B, cin, R, ksize, kpad, (int)train_precision(precision), s);
+  MDB_CUDA_CHECK(cudaStreamSynchronize(s));
   MDB_API_END
 }
 

@@ -3,6 +3,7 @@
 // kernels read hi + lo as one fp32 value and write what they compute back as a (hi, lo) pair.
 #include "backward.cuh"
 #include "gn_stats.cuh"
+#include "ptx.cuh"
 #include <stdexcept>
 #include <string>
 
@@ -43,15 +44,6 @@ __device__ __forceinline__ void pack8x(const float* x, uint4& hi, uint4& lo) {
   for (int j = 0; j < VEC; ++j) r[j] = x[j] - h[j];
   lo = pack8(r);
 }
-__device__ __forceinline__ float sigmoid_fast(float x) {
-  float t;
-  asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(0.5f * x));
-  return fmaf(0.5f, t, 0.5f);
-}
-__device__ __forceinline__ float dsilu(float y) {
-  const float s = sigmoid_fast(y);
-  return s * fmaf(y, 1.f - s, 1.f);
-}
 
 // grid.x for the staged, grid-stride kernels: the whole grid is ONE full wave of `target` = 148 x (resident blocks per
 // SM) blocks -- a 608-block launch at 2 blocks/SM (296 resident) spends a third, nearly empty wave on 16 blocks.
@@ -90,26 +82,9 @@ __device__ __forceinline__ void gn_stats_of(const GnBwdArgs& a, int b, int c, fl
   }
 }
 
-// dy[j] = da[j] * act'(y[j]) * dropout, xh[j] = normalised input
-__device__ __forceinline__ void gn_dy(const GnBwdArgs& a, const float* x, const float* da, const float* mean, const float* rstd,
-                                      const float* g, const float* be, long long e0, float* xh, float* dy) {
-  unsigned long long h0 = 0, h1 = 0;
-  if (a.drop_thresh > 0) { h0 = drop_hash64(a.seed, (unsigned long long)(e0 >> 2)); h1 = drop_hash64(a.seed, (unsigned long long)(e0 >> 2) + 1); }
-#pragma unroll
-  for (int j = 0; j < VEC; ++j) {
-    xh[j] = (x[j] - mean[j]) * rstd[j];
-    float d = da[j];
-    if (a.drop_thresh > 0) {
-      const unsigned r16 = (unsigned)(((j < 4 ? h0 : h1) >> (16 * (j & 3))) & 0xFFFFu);
-      d = r16 >= (unsigned)a.drop_thresh ? d * a.drop_scale : 0.f;
-    }
-    if (a.silu) d *= dsilu(fmaf(g[j], xh[j], be[j]));
-    dy[j] = d;
-  }
-}
-
 // Pass 1. Per element: h = 0.5*y straight from x (one FMA with folded constants), silu'(y) = t + 0.5*h*q with
-// t = (1+tanh h)/2, q = 1 - tanh^2 h; S2 is accumulated as sum(dy*x) and rebased to sum(dy*xhat) once per thread.
+// t = (1+tanh h)/2, q = 1 - tanh^2 h (X3: dsilu_of_half, accurate to the split operands' resolution); S2 is accumulated
+// as sum(dy*x) and rebased to sum(dy*xhat) once per thread.
 template <bool X3>
 __global__ void __launch_bounds__(256, 2) gn_bwd_reduce_kernel(GnBwdArgs a, int cv, int k) {
   constexpr int UNROLL = X3 ? 2 : 4;  // X3: twice the bytes per voxel in flight, within the 128-register budget
@@ -172,11 +147,15 @@ __global__ void __launch_bounds__(256, 2) gn_bwd_reduce_kernel(GnBwdArgs a, int 
 #pragma unroll
         for (int j = 0; j < VEC; ++j) {
           const float h = fmaf(x[j], hsc[j], hsh[j]);
-          float th;
-          asm("tanh.approx.f32 %0, %1;" : "=f"(th) : "f"(h));
-          const float q = fmaf(-th, th, 1.f);
-          const float t = fmaf(0.5f, th, 0.5f);
-          dy[j] *= fmaf(0.5f, h * q, t);
+          if constexpr (X3) {
+            dy[j] *= dsilu_of_half(h);
+          } else {
+            float th;
+            asm("tanh.approx.f32 %0, %1;" : "=f"(th) : "f"(h));
+            const float q = fmaf(-th, th, 1.f);
+            const float t = fmaf(0.5f, th, 0.5f);
+            dy[j] *= fmaf(0.5f, h * q, t);
+          }
         }
       }
 #pragma unroll

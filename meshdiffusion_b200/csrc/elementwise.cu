@@ -35,8 +35,9 @@ __device__ __forceinline__ float silu_f(float x) {
   asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(1.f + e));
   return x * r;
 }
-// x*sigmoid(x) = 0.5x(1 + tanh(x/2)) with the single-MUFU tanh.approx (rel. error 2^-11: below bf16 resolution);
-// halves the MUFU pressure of the bf16 GroupNorm+SiLU pass, which otherwise co-limits with HBM bandwidth.
+// x*sigmoid(x) = 0.5x(1 + tanh(x/2)) with the single-MUFU tanh.approx (rel. error 2^-11: below bf16 resolution, not
+// below the 2^-16 of a split-bf16 pair, so only the bf16 kernels use it); halves the MUFU pressure of the bf16
+// GroupNorm+SiLU pass, which otherwise co-limits with HBM bandwidth.
 __device__ __forceinline__ float silu_fast(float x) {
   float t;
   asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(0.5f * x));
@@ -452,6 +453,11 @@ void launch_transpose_vc(const void* in, long long ld, int c0, void* out, int B,
   if (tf32) transpose_vc_kernel<float><<<grid, block, 0, s>>>((const float*)in, ld, c0, (float*)out, V, C, ldo);
   else transpose_vc_kernel<__nv_bfloat16><<<grid, block, 0, s>>>((const __nv_bfloat16*)in, ld, c0, (__nv_bfloat16*)out, V, C, ldo);
   MDB_LAUNCH_CHECK();
+}
+void launch_transpose_vc_rows(const void* in, long long ld, int c0, void* out, int B, int V, int C, int x3, cudaStream_t s) {
+  if (!x3) { launch_transpose_vc(in, ld, c0, out, B, V, C, 0, s); return; }
+  launch_transpose_vc(in, 2 * ld, c0, out, B, V, C, 0, s, 2LL * V);
+  launch_transpose_vc(in, 2 * ld, (int)ld + c0, (__nv_bfloat16*)out + V, B, V, C, 0, s, 2LL * V);
 }
 
 // ------------------------------------------------------------------ time embedding MLP

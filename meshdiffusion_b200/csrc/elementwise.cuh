@@ -45,6 +45,8 @@ void launch_softmax_rows(float* s, long long rows, int L, int tf32, cudaStream_t
 // out[b][c][v] = in[b][v][c0 + c]
 void launch_transpose_vc(const void* in, long long ld_in, int c0, void* out, int B, int V, int C, int tf32,
                          cudaStream_t s, long long ld_out = 0);
+// the same for bf16 operand matrices of logical pitch ld; x3: (hi, lo) rows [ld hi | ld lo] -> [V hi | V lo] rows
+void launch_transpose_vc_rows(const void* in, long long ld, int c0, void* out, int B, int V, int C, int x3, cudaStream_t s);
 
 // temb path (ddpm_res64.py:132-136 + layers.py:542-556,680): act(temb)[B][4nf]
 void launch_temb(const float* labels, const float* w0, const float* b0, const float* w1, const float* b1, float* out,

@@ -674,9 +674,13 @@ __global__ void __launch_bounds__(kGemmThreads, 1) gemm_tc_kernel(const __grid_c
               }
               if (p.gnb_silu) {
                 const float h = fmaf(xv, kc.x, kc.y);
-                float th;
-                asm("tanh.approx.f32 %0, %1;" : "=f"(th) : "f"(h));
-                d *= fmaf(0.5f, h * fmaf(-th, th, 1.f), fmaf(0.5f, th, 0.5f));
+                if constexpr (X3) {
+                  d *= dsilu_of_half(h);
+                } else {
+                  float th;
+                  asm("tanh.approx.f32 %0, %1;" : "=f"(th) : "f"(h));
+                  d *= fmaf(0.5f, h * fmaf(-th, th, 1.f), fmaf(0.5f, th, 0.5f));
+                }
               }
               v[i] = d;
               q2[i] = d * fmaf(xv, kc.z, kc.w);

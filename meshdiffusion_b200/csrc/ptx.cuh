@@ -9,6 +9,16 @@
 
 namespace mdb {
 
+// SiLU derivative of y = 2h for split-bf16 operands: s = sigmoid(y) = 1 / (1 + 2^(-y log2 e)), silu'(y) = s (1 + y (1 - s)).
+// ex2.approx + rcp.approx (about 2^-22 relative each) keep it well below the 2^-17 resolution of a (hi, lo) bf16 pair; the
+// single-MUFU tanh.approx form the bf16 kernels use (2^-11) is only below bf16's.
+__device__ __forceinline__ float dsilu_of_half(float h) {
+  float e, s;
+  asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(h * -2.8853900817779268f));
+  asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(s) : "f"(1.f + e));
+  return s * fmaf(2.f * h, 1.f - s, 1.f);
+}
+
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }

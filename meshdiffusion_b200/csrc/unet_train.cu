@@ -425,9 +425,7 @@ void UNet::tape_attn(TensP x, TensP hn, TensP qkv, TensP S, TensP O, TensP out, 
     const size_t pp = parts(prec_);
     // transposed copy out[b][c][v] = in[b][v][c0 + c] of an operand matrix; X3: rows [ld hi | ld lo] -> [V hi | V lo]
     auto transpose = [x3, V](const void* in, long long ld, int c0, void* out, int B, int C_, cudaStream_t s) {
-      if (!x3) { launch_transpose_vc(in, ld, c0, out, B, V, C_, 0, s); return; }
-      launch_transpose_vc(in, 2 * ld, c0, out, B, V, C_, 0, s, 2LL * V);
-      launch_transpose_vc(in, 2 * ld, (int)ld + c0, (__nv_bfloat16*)out + V, B, V, C_, 0, s, 2LL * V);
+      launch_transpose_vc_rows(in, ld, c0, out, B, V, C_, x3 ? 1 : 0, s);
     };
     // P and dS: probabilities / logit gradients in the activation dtype at the start of rows of V fp32 slots -- a logical
     // pitch of 2V bf16, or V for X3 (whose [V hi | V lo] rows fill the slots)

@@ -13,6 +13,13 @@ from oracle import synth, unet_oracle
 
 pytestmark = pytest.mark.gpu
 
+# Gradient error against fp32 autograd, as relative L2 over all tensors and for the worst single tensor. Measured on one
+# B200 (1000 W power limit): global 3.9e-5 / 3.7e-5 / 4.9e-5, worst tensor 6.3e-5 / 9.4e-5 / 1.1e-4 (tiny res64, tiny
+# res128, full res64). The gates leave margin above that and stay well below the error one split kernel brings when it
+# drops its lo parts: zeroing them in the batch sum of the stem (global 2.0e-4, worst 1.8e-3) or the bias column sums
+# (worst 2.4e-3) passed the former gates of 1e-3 / 1e-2.
+GLOBAL_GATE, WORST_GATE = 2e-4, 1e-3
+
 
 def _cfg(name="res64", precision="bf16x3"):
     cfg = tiny_config(name, "bf16")
@@ -72,7 +79,7 @@ def test_x3_gradients_match_fp32_autograd(name):
     print(f"{name}: loss {loss:.6f} vs {ref_loss:.6f}; bf16x3 global rel-l2 {glob:.3e}, worst {worst[0]} {worst[1]:.3e}; "
           f"bf16 engine global {glob16:.3e}, worst {worst16[1]:.3e}; ratio {glob16 / glob:.1f}x")
     assert abs(loss - ref_loss) < 1e-3 * abs(ref_loss)
-    assert glob < 1e-3 and worst[1] < 1e-2
+    assert glob < GLOBAL_GATE and worst[1] < WORST_GATE
     assert glob * 10 <= glob16
 
 
@@ -126,7 +133,7 @@ def test_x3_res64_full_backward_vs_autograd():
     glob, worst = _errors(ours, ref)
     print(f"res64 full bf16x3: loss {loss:.6f} vs {ref_loss:.6f}; global rel-l2 {glob:.3e}, worst {worst[0]} {worst[1]:.3e}")
     assert abs(loss - ref_loss) < 1e-3 * abs(ref_loss)
-    assert glob < 1e-3 and worst[1] < 1e-2
+    assert glob < GLOBAL_GATE and worst[1] < WORST_GATE
 
 
 def test_x3_loss_curve_tracks_fp32_reference():
